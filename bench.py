@@ -2,6 +2,7 @@
 """Benchmark: ANPDistractor meta-train tasks/sec (BASELINE.json's metric) on N B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--precision tf32x3|tf32|fp32]
+                    [--dump-outputs DIR]
 
 One step = zero_grad + forward + loss + backward + (gradient all-reduce) + Adam on a synthetic
 Distractor-shaped meta-batch: 20 tasks per GPU (cfg/train/ANP_Distractor.yaml:10), 15 context
@@ -364,9 +365,16 @@ def run_b200_arm(args, rank, world, local_rank):
     if rank == 0:
         sampler.start()
     l0 = LIB.b200np_launch_count()
-    ms = timed(lambda i: run(resident[i % nbatch]), args.steps)
+    last = {}
+
+    def timed_step(i):
+        last["loss"] = run(resident[i % nbatch])
+    ms = timed(timed_step, args.steps)
     launches = launches_per_step * args.steps if args.graph else LIB.b200np_launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # before the e2e leg below trains the same model further
+        dump_outputs(args.dump_outputs, loss=last["loss"], params=flat.flat[:flat.n_live], grads=flat.grad)
 
     # end to end: pinned host inputs -> device every step, loss read back every step
     def e2e_step(i):
@@ -440,6 +448,15 @@ def run_b200_arm(args, rank, world, local_rank):
     line.update(extras)
     print(json.dumps(line), flush=True)
     finish()
+
+
+def dump_outputs(out_dir, **arrays):
+    """What the last timed step handed its caller, as float32 `<out_dir>/<name>.npy`: the loss, the flat live
+    parameters after the Adam update and the flat gradient they were updated with."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy().reshape(-1))
 
 
 def dropin_loop(args, dev, model_name, task, T, nc, nt):
@@ -671,7 +688,14 @@ def main():
                     help="run only the dominant-kernel timing (the command captured by `ncu --set full`)")
     ap.add_argument("--profile", action="store_true",
                     help="only the resident-input timed loop (for ncu launch lists); skips e2e / roofline / CPU legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's loss, updated parameters and gradient as "
+                         "DIR/<name>.npy (float32; same arguments, same inputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.roofline_only):
+        ap.error("--dump-outputs dumps the B200 arm's timed step: not with --impl reference* or --roofline-only")
     if args.scaling == "strong" and not args.tasks:
         ap.error("--scaling strong needs --tasks (the global meta-batch)")
     rank = int(os.environ.get("RANK", "0"))

@@ -109,17 +109,50 @@ def _reference_model_trainer():
     return mt.ModelTrainer
 
 
+class _RestatedTrainer:
+    """The training step the reference's ModelTrainer._train_iter takes (trainer/model_trainer.py:59-93), as bench.py's
+    e2e_dropin leg times it: zero_grad -> .to(device) of a host batch -> model -> calc_loss -> in-place
+    `losses += kl * beta` -> backward -> optimizer.step -> losses.item().  Lets the drop-in's training-loop contract
+    be checked without the reference tree."""
+
+    def _train_iter(self, it):
+        cfg = self.config
+        self.model.train()
+        self.optimizer.zero_grad()
+        ctx_x, qry_x, ctx_y, qry_y = (t.to(cfg.device)
+                                      for t in self.data.get_batch("train", cfg.tasks_per_batch, cfg.max_ctx_num))
+        pr_mu, pr_var, kl = self.model(ctx_x, ctx_y, qry_x)
+        losses = self.loss.calc_loss(pr_mu, pr_var, qry_y)
+        losses += kl * cfg.beta
+        losses.backward()
+        self.optimizer.step()
+        return losses.item()
+
+
 @needs_ref
 @pytest.mark.gpu
 @pytest.mark.parametrize("graphs", [False, True])
 @pytest.mark.parametrize("case", ["anp_distractor", "cnp_1d_max"])
 def test_unmodified_model_trainer_runs_on_the_dropin(case, graphs):
+    _check_trainer_on_the_dropin(_reference_model_trainer, case, graphs)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("graphs", [False, True])
+@pytest.mark.parametrize("case", ["anp_distractor", "cnp_1d_max"])
+def test_restated_training_loop_runs_on_the_dropin(case, graphs):
+    _check_trainer_on_the_dropin(lambda: _RestatedTrainer, case, graphs)
+
+
+def _check_trainer_on_the_dropin(trainer_class, case, graphs):
+    """Six `_train_iter` steps of `trainer_class()` on the drop-in modules with torch.optim.Adam and a context size
+    redrawn per step track the CPU oracle's loss; then one validation forward."""
     import importlib
     import types
     from b200np import engine
     from oracle import np_oracle
     engine.set_precision("tf32x3")
-    ModelTrainer = _reference_model_trainer()
+    ModelTrainer = trainer_class()
     method, task, agg, img_agg, extra, T, _, _ = CASES[case]
     cfg = make_config(method, task, T, agg, img_agg, device="cuda:0", **extra)
     cfg.max_ctx_num, cfg.lr = 15, 1e-3

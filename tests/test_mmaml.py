@@ -96,15 +96,29 @@ def _oracle_run(model, emb, dtype):
     return embeddings, logits.detach(), float(loss), pm, pe
 
 
+def _zero_gradients(p64):
+    """Names whose fp64 oracle gradient vanishes next to the largest one, and that largest norm.  These are conv biases in
+    front of batch normalisation with batch statistics, which removes any per-channel constant.  In fp32 their gradient
+    is rounding noise whose value depends on the CPU's math kernels, so, as in the GPU tests, it is bounded by the
+    gradient scale instead of being compared with the golden fingerprint of the reference's own noise."""
+    scale = max(float(v.grad.norm()) for v in p64.values())
+    return {k for k, v in p64.items() if float(v.grad.norm()) < 1e-9 * scale}, scale
+
+
 def test_oracle_matches_reference_golden(golden):
     model, emb = _build_models()
     embeddings, logits, loss, pm, pe = _oracle_run(model, emb, torch.float32)
+    _, _, _, pm64, pe64 = _oracle_run(model, emb, torch.float64)
     assert rel_l2(logits.numpy(), golden["logits"]) < 1e-5
     assert abs(loss - float(golden["loss"])) < 1e-5 * abs(float(golden["loss"]))
     for j, e in enumerate(embeddings):
         assert rel_l2(e.detach().numpy(), golden[f"embedding{j}"]) < 1e-5
-    for tag, ps in (("model", pm), ("emb", pe)):
+    for tag, ps, p64 in (("model", pm, pm64), ("emb", pe, pe64)):
+        zero, scale = _zero_gradients(p64)
         for k, ref in zip(golden[f"{tag}/grad_keys"], golden[f"{tag}/grad_fp"]):
+            if k in zero:
+                assert float(ps[k].grad.norm()) < 1e-5 * scale, (tag, k)
+                continue
             fp = fingerprint(ps[k].grad)
             assert abs(fp[2] - ref[2]) <= 2e-3 * ref[2] + 1e-9, (tag, k, fp, ref)
     with torch.no_grad():
@@ -215,11 +229,16 @@ def _oracle_meta_step(model, emb, dtype, second_order=True):
 def test_oracle_second_order_meta_step_matches_reference_golden(golden2):
     model, emb = _build_models()
     inner, outer, pred, pm, pe = _oracle_meta_step(model, emb, torch.float32)
+    _, _, _, pm64, pe64 = _oracle_meta_step(model, emb, torch.float64)
     np.testing.assert_allclose(inner, golden2["so/inner_losses"], rtol=2e-5)
     assert abs(outer - float(golden2["so/outer_loss"])) < 2e-5 * abs(float(golden2["so/outer_loss"]))
     assert rel_l2(pred.numpy(), golden2["so/pred"]) < 2e-5
-    for tag, ps in (("model", pm), ("emb", pe)):
+    for tag, ps, p64 in (("model", pm, pm64), ("emb", pe, pe64)):
+        zero, scale = _zero_gradients(p64)
         for k, ref in zip(golden2[f"so/{tag}/grad_keys"], golden2[f"so/{tag}/grad_fp"]):
+            if str(k) in zero:
+                assert float(ps[str(k)].grad.norm()) < 1e-5 * scale, (tag, k)
+                continue
             if ref[2] < 1e-6:
                 continue
             fp = fingerprint(ps[str(k)].grad)
