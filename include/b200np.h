@@ -363,14 +363,8 @@ int b200np_bbb_sample_kl_bwd(const float* dw, const float* dkl, const float* mu,
  * Diagnostics (tools/ only; never called on the product path).  They switch global state of the
  * library and are NOT thread-safe.
  *   b200np_debug_set_wgrad_waves   pixel chunks per weight-gradient launch = waves * resident CTAs
- *   b200np_debug_set_halo_flags    work-elimination bit mask for tools/halo_stalls.py (results become garbage)
- *   b200np_debug_set_halo_min_taps route tap convolutions with fewer taps to the gather kernel
- *   b200np_debug_set_halo_timing   device buffer [grid][8] of per-role stall-cycle counters (NULL = off)
  * ------------------------------------------------------------------------------------------ */
 void b200np_debug_set_wgrad_waves(int waves);
-void b200np_debug_set_halo_flags(int flags);
-void b200np_debug_set_halo_min_taps(int ntaps);
-void b200np_debug_set_halo_timing(long long* buf);
 
 /* ------------------------------------------------------------------------------------------
  * Multi-GPU.  SURVEY.md 8b sketched `b200np_comm_{init,allreduce_sum,allreduce_max,destroy}` wrappers over

@@ -126,35 +126,6 @@ def test_conv_block_ops(prec, cin, cout, hw, n):
         assert rel(from_nhwc(dx), x.grad) < tol
 
 
-def test_wgrad_halo_formulation_opt_in():
-    """The halo formulation of the 3x3 stride-1 (+ skip) weight gradient (csrc/tapwgrad_halo.cu) is selected per process
-    by B200NP_WGRAD_HALO=1: run the conv-block parity cases whose maps it covers (32x32 and 16x16) in a child process."""
-    import os
-    import subprocess
-    import sys
-    env = dict(os.environ, B200NP_WGRAD_HALO="1")
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-x", "-q", "-k",
-                        "conv_block and (64-64-64-2 or 64-64-32-3) and not fp32"], env=env, capture_output=True, text=True,
-                       timeout=600)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    assert " passed" in r.stdout and "4 passed" in r.stdout, r.stdout[-500:]
-
-
-def test_two_sm_halo_formulation_opt_in():
-    """The 2-SM (tcgen05.mma.cta_group::2, thread-block cluster of two) form of the TMA-fed halo convolution is selected
-    per process by B200NP_HALO_CG2=1 (experimental: correct, but paced by the peer-to-leader barrier relay -- DESIGN.md
-    finding 23): run the conv-block parity cases it covers in a child process."""
-    import os
-    import subprocess
-    import sys
-    env = dict(os.environ, B200NP_HALO_CG2="1")
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-x", "-q", "-k",
-                        "conv_block and (64-64-64-2 or 64-64-32-3) and not fp32"], env=env, capture_output=True, text=True,
-                       timeout=600)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    assert "4 passed" in r.stdout, r.stdout[-500:]
-
-
 def test_pools_and_flatten():
     ops = _ops()
     x = rnd(5, 64, 4, 4, seed=1)

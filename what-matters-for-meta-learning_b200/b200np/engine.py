@@ -73,9 +73,6 @@ _SIDE = {}
 # stream has the default (lowest) priority in eager mode; `optim.GraphedStep` captures on a stream of MAIN_PRIORITY.
 MAIN_PRIORITY, DECODER_PRIORITY, WGRAD_PRIORITY = -2, -1, 0
 USE_PRIORITIES = os.environ.get("B200NP_PRIO", "1") != "0"
-FORK = os.environ.get("B200NP_FORK", "early")   # where the decoder branch forks: early | late (see the forward)
-STEM_GEMM = os.environ.get("B200NP_STEM_GEMM", "1") != "0"       # stems without a tcgen05 stem kernel: im2col + GEMM
-W0_IMPLICIT = os.environ.get("B200NP_W0_IMPLICIT", "1") != "0"   # encoder_w0's 3x3 convs as implicit-convolution GEMMs
 
 
 # Called at the start of every CNN trunk's backward with the data pointer of the trunk's first parameter.  By then every
@@ -127,7 +124,7 @@ class TrunkFn(Function):
         # Stems the tcgen05 stem kernel does not cover (3-channel tasks: 5x5 over RGB, K = 75) in the tensor-core modes:
         # im2col of the thin NCHW input + the tcgen05 GEMM with a fused bias + ReLU epilogue, and dW = dY^T col in the
         # backward -- the CUDA-core direct convolution and its weight gradient were 22 % of the ShapeNet3D step
-        stem_cols = [] if (STEM_GEMM and prec != PREC_FP32_SIMT and bits0 is None) else None
+        stem_cols = [] if (prec != PREC_FP32_SIMT and bits0 is None) else None
         for im, n in zip(imgs, Ns):
             if stem_cols is not None:
                 R, K = c1w.shape[2], c1w.shape[1] * c1w.shape[2] * c1w.shape[3]
@@ -266,13 +263,12 @@ class EncoderW0Fn(Function):
             x2 = ops.conv_fwd(x1, wd2, b2, 2, ACT_RELU, prec)
             x3, pidx = ops.maxpool2x2_fwd(x2)
             x4 = ops.conv_fwd(x3, wd5, b5, 2, ACT_RELU, prec)
-            col2 = col5 = None
-        elif W0_IMPLICIT:
+        else:
             # 32 -> 48 and 48 -> 64 channels do not fill the 64 x 64 tap-convolution tiles: the tcgen05 GEMM with a VIRTUAL
             # im2col operand (b200np_gemm_desc.conv_operand: k = tap*C + ci, gathered as 16-byte words while the operand
             # is staged) and a fused bias + ReLU epilogue -- no column matrix is written or read (it was 354 MB for the
             # 32 -> 48 layer of 300 images, written once and read twice per step)
-            wd2 = wd5 = col2 = col5 = None
+            wd2 = wd5 = None
             w2, w5 = ops.conv_weight_tapmajor(w2), ops.conv_weight_tapmajor(w5)      # [Cout, 9*Cin], tap-major
             M2, K2 = N * (H // 4) * (W // 4), w2.shape[1]
             x2 = ops.empty((N, H // 4, W // 4, w2.shape[0]), imgs[0])
@@ -283,32 +279,20 @@ class EncoderW0Fn(Function):
             x4 = ops.empty((N, H // 16, W // 16, w5.shape[0]), imgs[0])
             ops.gemm(_p(x3), _p(w5), _p(x4), M5, w5.shape[0], K5, K5, 1, 1, K5, w5.shape[0], bias=_p(b5), act=ACT_RELU,
                      prec=prec, conv=(1, H // 8, W // 8, x3.shape[-1]))
-        else:
-            # B200NP_W0_IMPLICIT=0: explicit im2col (k = ci*9 + tap, the flattening of torch's weight) + the tcgen05 GEMM
-            wd2 = wd5 = None
-            col2 = ops.im2col3x3s2(x1)
-            x2 = ops.empty((N, H // 4, W // 4, w2.shape[0]), imgs[0])
-            ops.gemm(_p(col2), _p(w2), _p(x2), col2.shape[0], w2.shape[0], col2.shape[1], col2.shape[1], 1, 1,
-                     col2.shape[1], w2.shape[0], bias=_p(b2), act=ACT_RELU, prec=prec)
-            x3, pidx = ops.maxpool2x2_fwd(x2)
-            col5 = ops.im2col3x3s2(x3)
-            x4 = ops.empty((N, H // 16, W // 16, w5.shape[0]), imgs[0])
-            ops.gemm(_p(col5), _p(w5), _p(x4), col5.shape[0], w5.shape[0], col5.shape[1], col5.shape[1], 1, 1,
-                     col5.shape[1], w5.shape[0], bias=_p(b5), act=ACT_RELU, prec=prec)
         outs, off = [], 0
         for n in Ns:
             outs.append(ops.nhwc_to_nchw_flat(x4[off:off + n]))
             off += n
         ctx.prec, ctx.Ns, ctx.imgs = prec, Ns, img_all
         ctx.first_param_ptr = w0.data_ptr()
-        ctx.saved = (x1, x2, x3, x4, pidx, wd2, wd5, tuple(w0.shape), col2, col5, w2, w5)
+        ctx.saved = (x1, x2, x3, x4, pidx, wd2, wd5, tuple(w0.shape), w2, w5)
         return tuple(outs)
 
     @staticmethod
     def backward(ctx, *douts):
         prec, Ns = ctx.prec, ctx.Ns
         _pre_trunk_backward(ctx.first_param_ptr)
-        x1, x2, x3, x4, pidx, wd2, wd5, w0_shape, col2, col5, w2, w5 = ctx.saved
+        x1, x2, x3, x4, pidx, wd2, wd5, w0_shape, w2, w5 = ctx.saved
         d4 = torch.empty_like(x4)
         off = 0
         for n, do in zip(Ns, douts):
@@ -320,7 +304,7 @@ class EncoderW0Fn(Function):
             d2 = ops.maxpool2x2_bwd(d3, pidx, x2)
             dw2, db2, _ = ops.conv_wgrad(x1, d2, 3, 2, prec)
             d1 = ops.conv_dgrad(d2, wd2, x1.shape, 2, prec, mask_src=x1)
-        elif col2 is None:
+        else:
             def conv_bwd(x_in, wt, dy, mask):     # wt: tap-major [Cout, 9*Cin]; x_in NHWC, the conv's input
                 Co, K = wt.shape
                 M = dy.numel() // Co
@@ -334,19 +318,6 @@ class EncoderW0Fn(Function):
             dw5, db5, d3 = conv_bwd(x3, w5, d4, None)
             d2 = ops.maxpool2x2_bwd(d3, pidx, x2)
             dw2, db2, d1 = conv_bwd(x1, w2, d2, x1)
-        else:
-            def conv_bwd(col, w, dy, x_shape, mask):
-                M, K = col.shape
-                Co = w.shape[0]
-                dw = ops.empty(tuple(w.shape), w)
-                ops.gemm(_p(dy), _p(col), _p(dw), Co, K, M, 1, Co, K, 1, K, prec=prec)             # dW = dY^T col
-                db = ops.colsum(dy, M, Co, Co)
-                dcol = ops.empty((M, K), dy)
-                ops.gemm(_p(dy), _p(w), _p(dcol), M, K, Co, Co, 1, K, 1, K, prec=prec)             # dcol = dY W
-                return dw, db, ops.col2im3x3s2(dcol, x_shape, mask=mask)
-            dw5, db5, d3 = conv_bwd(col5, w5, d4, x3.shape, None)
-            d2 = ops.maxpool2x2_bwd(d3, pidx, x2)
-            dw2, db2, d1 = conv_bwd(col2, w2, d2, x1.shape, x1)
         dw0, db0 = ops.conv_small_wgrad(ctx.imgs, d1, w0_shape, prec)
         return (None, None) + (None,) * len(Ns) + (dw0, db0, dw2, db2, dw5, db5)
 
@@ -613,23 +584,13 @@ def _forward_resnet_family(m, ctx_x, ctx_y, tgt_x):
     C, H, W = m.img_channels, m.img_size[0], m.img_size[1]
     tgt_imgs = tgt_x.reshape(T * nt, C, H, W).contiguous()
     dec_params = _trunk_params(m.decoder)
-    side = x_dec = None
-
-    def fork_decoder():
-        nonlocal side, x_dec, main
+    side = None
+    if OVERLAP >= 1 and nc:
         main = torch.cuda.current_stream()
         side = _side_stream(("decoder", main.cuda_stream), DECODER_PRIORITY)
         side.wait_stream(main)
         with torch.cuda.stream(side):
             (x_dec,) = TrunkFn.apply(m.img_agg, PRECISION, 1, tgt_imgs, *dec_params)
-    main = None
-    # Where the decoder branch forks: before the encoder CNN (default), or after it is enqueued ("late": the decoder
-    # CNN's big kernels then run beside the latency-bound dense / FAVOR+ chain instead of beside the encoder CNN).
-    # Measured on ANPDistractor: late 8.155 ms/step, early 8.12 -- the attention section runs alone less (FAVOR+ forward
-    # 0.12 -> 0.07 ms solo, tools/timeline_gaps.py) but the two CNNs' small-map layers lose their overlap.
-    late_fork = OVERLAP >= 1 and nc and FORK == "late"
-    if OVERLAP >= 1 and nc and not late_fork:
-        fork_decoder()
     if nc:
         ctx_imgs = ctx_x.reshape(T * nc, C, H, W).contiguous()
         lab = ctx_y.reshape(T * nc, -1).contiguous()
@@ -638,14 +599,10 @@ def _forward_resnet_family(m, ctx_x, ctx_y, tgt_x):
         enc = _trunk_params(m.img_encoder)
         if m.attention:
             x_ctx, x_tgt = TrunkFn.apply(m.img_agg, PRECISION, 2, ctx_imgs, tgt_imgs, *enc)
-            if late_fork:
-                fork_decoder()
         else:
             if m.agg_mode not in ("mean", "max", "baco"):
                 raise TypeError("agg_mode is not applicable for CNP, choose from ['mean', 'max', 'baco']")
             (x_ctx,) = TrunkFn.apply(m.img_agg, PRECISION, 1, ctx_imgs, *enc)
-            if late_fork:
-                fork_decoder()
         cf = _lin(ACT_RELU, x_ctx, lab, m.task_encoder[0])
         cf = _lin(ACT_RELU, cf, None, m.task_encoder[2])
         cf = _lin(ACT_RELU, cf, None, m.task_encoder[4])

@@ -85,9 +85,6 @@ SIGNATURES = {
     "b200np_bbb_sample_kl_fwd": (_i, [_p, _p, _p, _f, _f, _p, _p, _p, _ll, _p]),
     "b200np_bbb_sample_kl_bwd": (_i, [_p, _p, _p, _p, _p, _p, _f, _f, _p, _p, _ll, _p]),
     "b200np_debug_set_wgrad_waves": (None, [_i]),
-    "b200np_debug_set_halo_flags": (None, [_i]),
-    "b200np_debug_set_halo_min_taps": (None, [_i]),
-    "b200np_debug_set_halo_timing": (None, [_p]),
 }
 
 

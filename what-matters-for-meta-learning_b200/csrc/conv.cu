@@ -1,14 +1,8 @@
 // C ABI of the channel-dense NHWC convolutions: builds tap tables (tapconv.cuh) for forward,
 // data-gradient and weight-gradient and dispatches to the tcgen05 kernels (64-channel layers) or
 // the CUDA-core kernels (fp32 validation mode; 32/48-channel layers of encoder_w0).
-#include <cstdlib>
-
 #include "tapconv.cuh"
 #include "umma.cuh"
-
-#ifndef WGRAD_HALO_DEFAULT
-#define WGRAD_HALO_DEFAULT true
-#endif
 
 using namespace b200np;
 
@@ -209,13 +203,9 @@ extern "C" int b200np_conv_dgrad(const float* dy, const float* wd, float* dx, co
   return B200NP_OK;
 }
 
-// The halo formulation of the 3x3 stride-1 weight gradient (tapwgrad_halo.cu).  B200NP_WGRAD_HALO=0 keeps the gather kernel.
-static bool wgrad_halo_enabled() {
-  static const bool on = [] { const char* e = getenv("B200NP_WGRAD_HALO"); return e ? e[0] != '0' : WGRAD_HALO_DEFAULT; }();
-  return on;
-}
+// Pixel chunks of the halo formulation of a 64->64 3x3 weight gradient (tapwgrad_halo.cu); 0 where it does not apply.
 static int halo_chunks_for(int N, int OH, int OW, int Cin, int Cout, int R, int stride) {
-  if (!(wgrad_halo_enabled() && Cin == 64 && Cout == 64 && R == 3)) return 0;
+  if (!(Cin == 64 && Cout == 64 && R == 3)) return 0;
   return stride == 1 ? tapwgrad_halo_chunks(N, OH, OW) : stride == 2 ? tapwgrad_halo_s2_chunks(N, OH, OW) : 0;
 }
 

@@ -384,11 +384,7 @@ __global__ void __launch_bounds__(128, 4)
 
 int stem_wgrad_chunks(long long M) {
   // CTAs per SM over the whole launch (4 are resident at a time); every CTA leaves a 16 KB partial for the reducer
-  static const int per_sm = [] {
-    const char* e = getenv("B200NP_STEM_WGRAD_CTAS");
-    const int v = (e && e[0]) ? atoi(e) : 4;   // one resident wave; 8: +38 us per step in reducer traffic, 2: tail
-    return v >= 1 && v <= 32 ? v : 4;
-  }();
+  constexpr int per_sm = 4;   // one resident wave; 8: +38 us per step in reducer traffic, 2: tail
   long long want = (long long)per_sm * kNumSMs, maxc = ceil_div(M, 64);
   if (want > maxc) want = maxc;
   return (int)(want < 1 ? 1 : want);

@@ -18,13 +18,22 @@
 //     absolute-address swizzle -- verified on B200 by tools/probe.)
 //
 // Weights arrive pre-split (hi/lo) and pre-swizzled from b200np_pack_conv_weight, one 16 KB K-block
-// (tap, channel half) per cp.async.bulk into a ring that takes whatever shared memory the stages leave.
+// (tap, channel half) per cp.async.bulk into a ring of 3, 4 or 6 slots.
 //
-// Persistent, warp-specialised CTA (one per SM), tiles round-robin:
-//   warps 0-7   plane producers (gather + split + store), one stage = one channel half of one tile; eight
-//               warps because the producers are instruction-issue bound, not memory bound (ncu)
-//   warp  8     weight producer (one lane issues bulk copies); also owns the TMEM allocation
-//   warp  9     MMA issuer (one lane)
+// Persistent, warp-specialised CTA (one per SM), tiles round-robin, one stage = one channel half of one tile:
+//   warp  14    plane loader: ONE cp.async.bulk.tensor per plane (HaloTma) lands the raw fp32 pixels in the `hi`
+//               plane of the stage -- no global-load / address arithmetic in any thread, out-of-bounds pixels
+//               zero-filled by the copy engine;
+//   warps 0-7   split warps: shared memory -> shared memory, one LDS + one STS per 16 bytes.  fp32-grade mode: the
+//               landed raw plane is used as the `hi` operand as it is -- the tensor core truncates fp32 to tf32 --
+//               and only lo = x - trunc_tf32(x) is written to the `lo` plane; single-pass mode: the landed values
+//               are rounded to nearest in place.  (Producers that gathered with global loads spent LDG + address
+//               decode + two STS per 16 bytes; the L1 data pipe, which the tensor core's operand reads share, was
+//               95 % busy: 0.57 ms against 0.535 ms on the layer1 conv2 + skip launch.)
+//   warp  8     weight loader (one lane issues bulk copies); also owns the TMEM allocation
+//   warp  9     MMA issuer with the tap loop unrolled (9 or 10 taps): every per-tap descriptor word is a
+//               loop-invariant uniform register, and the `weights landed` probe of tap t+1 is issued before the
+//               MMAs of tap t, so its ~90-cycle latency hides behind the issue of eight MMAs
 //   warps 10-13 epilogue (TMEM -> registers -> bias / ReLU mask / activation -> NHWC global)
 // Two accumulator sets in TMEM let the epilogue of tile i overlap the MMAs of tile i+1.
 //
@@ -33,7 +42,6 @@
 // A_hi x [B_hi;B_lo] (N = 128, 64 cycles) yields hi*hi (columns 0-63) and hi*lo (64-127), then A_lo x B_hi
 // (N = 64) adds the other cross term into columns 64-127.  Accumulator blocks of 128 columns rotate (kRot)
 // to bound the bias of the tensor core's truncating fp32 accumulation; the epilogue sums them.
-#include <cstdlib>
 
 #include "tapconv.cuh"
 #include "tma.cuh"
@@ -43,29 +51,16 @@ namespace b200np {
 
 using namespace umma;
 
-// Diagnostic hooks (tools/halo_stalls.py): per-role blocked-cycle counters; nullptr in normal operation.
-static long long* g_halo_dbg = nullptr;
-__device__ float g_zero_line[32];  // 128 bytes of zeros: what padded / unused producer tasks load
-
-static int g_halo_min_taps = 1;
-static int g_halo_flags = 0;   // diagnostics (results are garbage): 1 = no weight copies, 2 = no plane loads/stores,
-                               // 4 = no epilogue stores / mask loads, 8 = no cross-term MMAs, 16 = no MMAs
-extern "C" void b200np_debug_set_halo_flags(int f) { g_halo_flags = f; }
-extern "C" void b200np_debug_set_halo_min_taps(int n) { g_halo_min_taps = n; }
-extern "C" void b200np_debug_set_halo_timing(long long* buf) { g_halo_dbg = buf; }
-
 namespace {
 
 constexpr int kTileRows = 16, kTileCols = 8;
 constexpr int kMaxPlanes = 5;
-constexpr bool kPipeProducers = false;  // two register buffers per producer thread: measured slower (register pressure)
-constexpr int kMaxBStages = 10;
+constexpr int kMaxBStages = 6;                           // deepest weight ring (launch_halo picks 3, 4 or 6)
 constexpr int kRot = 2;                                  // rotating accumulator blocks per accumulator set
 constexpr uint32_t kBSlotBytes = 2 * kBBytes;            // hi + lo = 16 KB
-constexpr int kProducerWarps = 8, kProducerThreads = 32 * kProducerWarps;
-constexpr int kWeightWarp = kProducerWarps, kMmaWarp = kProducerWarps + 1, kEpiWarp0 = kProducerWarps + 2;
-constexpr int kThreads = 32 * (kProducerWarps + 2 + 4);
-constexpr int kSlotsPerPass = kProducerThreads / 8;      // slots covered by one pass of the producers
+constexpr int kSplitWarps = 8, kSplitThreads = 32 * kSplitWarps;
+constexpr int kWeightWarp = 8, kMmaWarp = 9, kEpiWarp0 = 10, kTmaWarp = 14;
+constexpr int kThreads = 32 * (kTmaWarp + 1);
 constexpr uint32_t kSmemBudget = 227 * 1024;
 
 struct Plane {
@@ -92,11 +87,9 @@ struct HaloArgs {
   int tiles_x, tiles_total;
   uint32_t plane_bytes, stage_bytes, b_off, bar_off;
   int nb;                  // weight ring depth
-  int dbg_flags;
-  long long* dbg;          // optional [gridDim.x][8] stall-cycle counters
 };
 
-// Tensor maps of the planes (TMA-fed kernel): one 4-D map per plane over its source tensor -- [channel][x][y][image],
+// Tensor maps of the planes: one 4-D map per plane over its source tensor -- [channel][x][y][image],
 // for a stride-2 parity plane the view x[2j + px][2i + py] (base shifted, strides doubled) -- with a box of 32 channels
 // x HC x HR x 1 and SWIZZLE_128B, so that ONE bulk tensor copy lands a whole plane of a channel half in exactly the
 // slot layout the UMMA descriptors expect; out-of-bounds pixels arrive as zeros (= the convolution's padding).
@@ -119,12 +112,6 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t by
                "l"(src), "r"(bytes), "r"(smem_u32(bar))
                : "memory");
 }
-__device__ __forceinline__ void mbar_wait_timed(uint64_t* bar, uint32_t parity, long long& acc, bool timed) {
-  if (!timed) { mbar_wait(bar, parity); return; }
-  const long long t0 = clock64();
-  mbar_wait(bar, parity);
-  acc += clock64() - t0;
-}
 
 struct Ring {
   int idx = 0;
@@ -134,11 +121,11 @@ struct Ring {
   }
 };
 
-// ===================== epilogue (shared by the register-staged and the TMA-fed kernel) =====================
+// ===================== epilogue =====================
 // warps kEpiWarp0 .. kEpiWarp0+3: TMEM -> registers -> bias / ReLU gates / activation -> NHWC global
-template <bool X3, bool DBG>
+template <bool X3>
 __device__ __forceinline__ void halo_epilogue(const HaloArgs& h, uint64_t* acc_full, uint64_t* acc_empty,
-                                              uint32_t tmem_base, int warp, int lane, int dflags, long long* dbgp) {
+                                              uint32_t tmem_base, int warp, int lane) {
   const TapConvArgs& a = h.t;
   constexpr uint32_t kAccCols = X3 ? 256u : 128u;
   constexpr uint32_t kBlkCols = X3 ? 128u : 64u;
@@ -152,7 +139,6 @@ __device__ __forceinline__ void halo_epilogue(const HaloArgs& h, uint64_t* acc_f
   const int m = q * 32 + lane;                         // accumulator row = output pixel of the tile
   int acc_set = 0;
   uint32_t acc_phase = 0;
-  long long w_e = 0;
   const int kb_total = 2 * ntaps;
   const int blocks_used = ncls > 1 ? 1 : (kb_total < kRot ? kb_total : kRot);
   for (int tile = blockIdx.x; tile < h.tiles_total; tile += gridDim.x) {
@@ -182,7 +168,7 @@ __device__ __forceinline__ void halo_epilogue(const HaloArgs& h, uint64_t* acc_f
     const int d_oy = ncls > 1 ? h.cls_oy[cls] : a.dst_oy, d_ox = ncls > 1 ? h.cls_ox[cls] : a.dst_ox;
     const long long off =
         (((long long)n * a.dstH + (long long)oy * a.dst_s + d_oy) * a.dstW + (long long)ox * a.dst_s + d_ox) * 64;
-    mbar_wait_timed(acc_full + set, acc_phase, w_e, dbgp != nullptr);
+    mbar_wait(acc_full + set, acc_phase);
     tc_fence_after();
     const uint32_t taddr = tmem_base + set * set_stride + (static_cast<uint32_t>(q * 32) << 16);
 #pragma unroll
@@ -216,7 +202,7 @@ __device__ __forceinline__ void halo_epilogue(const HaloArgs& h, uint64_t* acc_f
       const uint32_t mword = hf ? mw1 : mw0;             // 32 ReLU gates
       uint32_t gates = 0u;                               // (output > 0) of this thread's 32 channels
       // float-mask variant: all eight loads are issued before the first use (one exposed latency, not eight)
-      const bool fmask = !a.mask_bits && a.mask && !(dflags & 4);
+      const bool fmask = !a.mask_bits && a.mask;
       float4 mk8[8];
       if (fmask) {
 #pragma unroll
@@ -246,7 +232,7 @@ __device__ __forceinline__ void halo_epilogue(const HaloArgs& h, uint64_t* acc_f
         if (a.act == B200NP_ACT_RELU) {
           o.x = fmaxf(o.x, 0.f); o.y = fmaxf(o.y, 0.f); o.z = fmaxf(o.z, 0.f); o.w = fmaxf(o.w, 0.f);
         }
-        if (!(dflags & 4) || o.x == 12345.678f) *reinterpret_cast<float4*>(a.dst + off + c) = o;
+        *reinterpret_cast<float4*>(a.dst + off + c) = o;
         gates |= (uint32_t)((o.x > 0.f) | ((o.y > 0.f) << 1) | ((o.z > 0.f) << 2) | ((o.w > 0.f) << 3)) << (4 * qq);
       }
       if (a.relu_bits) a.relu_bits[(off >> 6) * 2 + hf] = gates;
@@ -255,304 +241,7 @@ __device__ __forceinline__ void halo_epilogue(const HaloArgs& h, uint64_t* acc_f
     if (ncls > 1) acc_phase ^= 1;                      // every class set is used once per tile
     else if (++acc_set == 2) { acc_set = 0; acc_phase ^= 1; }
   }
-  if (dbgp && warp == kEpiWarp0 && lane == 0) dbgp[blockIdx.x * 8 + 7] = w_e;
 }
-
-// MAXT = 16-byte chunk tasks per producer thread and stage (ceil(total_slots / 32))
-// DBG: diagnostic build (stall counters, work-elimination flags); the production build compiles them out
-template <bool X3, int MAXT, bool DBG>
-__global__ void __launch_bounds__(kThreads, 1) tapconv_halo_kernel(const HaloArgs h) {
-  constexpr uint32_t kBSlot = b_slot_bytes<X3>();
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + h.bar_off);
-  uint64_t* a_full = bars;                  // [a_stages] producers -> MMA            (count 256)
-  uint64_t* a_empty = bars + 2;             // [a_stages] MMA commit -> producers     (count 1)
-  uint64_t* acc_full = bars + 4;            // [4] MMA commit -> epilogue             (count 1)
-  uint64_t* acc_empty = bars + 8;           // [4] epilogue -> MMA                    (count 128)
-  uint64_t* b_full = bars + 12;             // [nb] bulk copy tx -> MMA               (count 1 + tx)
-  uint64_t* b_empty = b_full + kMaxBStages; // [nb] MMA commit -> weight warp         (count 1)
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(b_empty + kMaxBStages);
-  const int nb = h.nb, a_stages = h.a_stages;
-
-  const TapConvArgs& a = h.t;
-  const int dflags = DBG ? h.dbg_flags : 0;
-  long long* const dbgp = DBG ? h.dbg : nullptr;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  constexpr uint32_t kAccCols = X3 ? 256u : 128u;       // columns per accumulator set: kRot blocks of 128 | 64
-  constexpr uint32_t kTmemCols = 2 * kAccCols;
-  // class mode (h.ncls > 1): one accumulator set per output class, a single block each (K <= 4 taps x 64, no
-  // rotation needed): 4 x 128 | 64 columns = the same TMEM allocation
-  constexpr uint32_t kBlkCols = X3 ? 128u : 64u;
-  const int ncls = h.ncls;
-  const uint32_t set_stride = ncls > 1 ? kBlkCols : kAccCols;
-
-  if (tid == 0) {
-    for (int s = 0; s < a_stages; ++s) { mbar_init(a_full + s, kProducerThreads); mbar_init(a_empty + s, 1); }
-    for (int s = 0; s < nb; ++s) { mbar_init(b_full + s, 1); mbar_init(b_empty + s, 1); }
-    for (int s = 0; s < 4; ++s) { mbar_init(acc_full + s, 1); mbar_init(acc_empty + s, 128); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == kWeightWarp) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(kTmemCols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const int ntaps = a.ntaps;
-
-  if (warp < kProducerWarps) {
-    // ===================== plane producers =====================
-    // Thread = fixed 16-byte chunk c of slots s0, s0+32, s0+64, ...  Which plane / row / column each of
-    // those slots is does not depend on the tile: it is decoded once into `meta` (no division in the loop;
-    // with one or two producer warps per scheduler, address arithmetic is the producers' critical path).
-    Ring st;
-    long long dbg_a = 0;
-    const long long dbg_t0 = clock64();
-    const int c = tid & 7, s0 = tid >> 3;
-    // meta[i]: source-pixel offset of the task relative to the tile origin, packed
-    //   bits 0-7 by + 64, bits 8-15 bx + 64   (source row = oy0 * scale + by, column = ox0 * scale + bx)
-    //   bit 16 source tensor (0 = a.src[0], 1 = the fused skip source), bit 17 = task exists
-    // Everything else the address needs (pointer, height, width, scale of the two sources) is warp-uniform and
-    // stays in registers.  The loop body is branch-free: padding and non-existent tasks load a line of zeros,
-    // so the MAXT loads of a stage have distinct destination registers and issue back to back.  (The first
-    // version indexed the plane table in the constant bank per task and branched around every load: ~45
-    // dependent instructions per task, 1.06 ms for the four-plane stride-2 forward conv; now 0.79 ms.)
-    int meta[MAXT];
-#pragma unroll
-    for (int i = 0; i < MAXT; ++i) {
-      const int slot = s0 + i * kSlotsPerPass;
-      meta[i] = 0;
-      for (int p = 0; p < h.nplanes; ++p) {
-        const Plane& P = h.pl[p];
-        const int local = slot - P.slot0;
-        if (local >= 0 && local < P.nslots) {
-          const int hy = local / P.HC, hx = local - hy * P.HC;
-          if (hy < P.HR) {
-            const int by = (P.dy_min + hy) * P.scale + P.py, bx = (P.dx_min + hx) * P.scale + P.px;
-            meta[i] = (by + 64) | ((bx + 64) << 8) | ((P.src == a.src[0] && P.scale == a.in_s[0] ? 0 : 1) << 16) | (1 << 17);
-          }
-        }
-      }
-    }
-    const float* const src0 = a.src[0];
-    const float* const src1 = a.src[1] ? a.src[1] : a.src[0];
-    const int H0 = a.srcH[0], W0 = a.srcW[0], sc0 = a.in_s[0];
-    const int H1 = a.src[1] ? a.srcH[1] : H0, W1 = a.src[1] ? a.srcW[1] : W0, sc1 = a.src[1] ? a.in_s[1] : sc0;
-    auto load_stage = [&](int tile, int half, float4 (&v)[MAXT]) {
-      const int xt = tile % h.tiles_x, rb = tile / h.tiles_x;
-      const int r0 = rb * kTileRows;
-      const int n = r0 / a.OH, oy0 = r0 - n * a.OH, ox0 = xt * kTileCols;
-      const int coff = half * 32 + c * 4;
-      const float* const img0 = src0 + (long long)n * H0 * W0 * 64 + coff;
-      const float* const img1 = src1 + (long long)n * H1 * W1 * 64 + coff;
-      const int oy0a = oy0 * sc0 - 64, ox0a = ox0 * sc0 - 64, oy0b = oy0 * sc1 - 64, ox0b = ox0 * sc1 - 64;
-#pragma unroll
-      for (int i = 0; i < MAXT; ++i) {
-        const int mt = meta[i];
-        const bool second = (mt >> 16) & 1;
-        const int iy = (second ? oy0b : oy0a) + (mt & 0xff), ix = (second ? ox0b : ox0a) + ((mt >> 8) & 0xff);
-        const int sH = second ? H1 : H0, sW = second ? W1 : W0;
-        const bool ok = ((mt >> 17) & 1) && (unsigned)iy < (unsigned)sH && (unsigned)ix < (unsigned)sW && !(dflags & 2);
-        const float* const img = second ? img1 : img0;
-        v[i] = ldg4(ok ? img + (iy * sW + ix) * 64 : g_zero_line);
-      }
-    };
-    auto store_stage = [&](float4 (&v)[MAXT]) {
-      mbar_wait_timed(a_empty + st.idx, st.phase ^ 1, dbg_a, dbgp != nullptr);
-      uint8_t* plane_hi = smem + st.idx * h.stage_bytes;
-      uint8_t* plane_lo = plane_hi + h.plane_bytes;
-#pragma unroll
-      for (int i = 0; i < MAXT; ++i) {
-        const int slot = s0 + i * kSlotsPerPass;
-        // stage bases are 1024-aligned, so the absolute-address swizzle phase of a slot is slot & 7
-        if (slot < h.total_slots && !(dflags & 2))
-          split_store(plane_hi, plane_lo, (uint32_t)(slot * 128 + ((c ^ (slot & 7)) << 4)), v[i], X3);
-      }
-      fence_proxy_async();
-      mbar_arrive(a_full + st.idx);
-      st.advance(a_stages);
-    };
-    if (kPipeProducers && MAXT <= 10) {
-      // Two register buffers: the loads of the NEXT stage are in flight while this one is converted and
-      // stored.  (With one buffer a stage cost a full DRAM round trip plus the stores, ~6K cycles, and the
-      // producers -- not the tensor core -- set the pace of the kernel.)
-      float4 v0[MAXT], v1[MAXT];
-      int tile = blockIdx.x;
-      if (tile < h.tiles_total) load_stage(tile, 0, v0);
-      for (; tile < h.tiles_total; tile += gridDim.x) {
-        load_stage(tile, 1, v1);
-        store_stage(v0);
-        if (tile + (int)gridDim.x < h.tiles_total) load_stage(tile + gridDim.x, 0, v0);
-        store_stage(v1);
-      }
-    } else {
-      float4 v[MAXT];
-      for (int tile = blockIdx.x; tile < h.tiles_total; tile += gridDim.x)
-        for (int half = 0; half < 2; ++half) {
-          load_stage(tile, half, v);
-          store_stage(v);
-        }
-    }
-    if (dbgp && tid == 0) { dbgp[blockIdx.x * 8 + 0] = dbg_a; dbgp[blockIdx.x * 8 + 1] = clock64() - dbg_t0; }
-  } else if (warp == kWeightWarp) {
-    // ===================== weight producer =====================
-    // (all lanes run the loop, the elected one issues: the bulk copy also takes uniform-register operands)
-    const bool leader = elect_one_sync();
-    {
-      Ring bs;
-      long long dbg_b = 0;
-      for (int tile = blockIdx.x; tile < h.tiles_total; tile += gridDim.x) {
-        for (int half = 0; half < 2; ++half) {
-          for (int t = 0; t < ntaps; ++t) {
-            const Tap tp = a.taps[t];
-            const float* src = h.bp[tp.src] + ((long long)half * h.nslabs[tp.src] + tp.slab) * (kBSlotBytes / 4);
-            if (!(dflags & 32)) mbar_wait_timed(b_empty + bs.idx, bs.phase ^ 1, dbg_b, dbgp != nullptr);
-            if (leader && !(dflags & 64)) {
-              if (dflags & 1) {
-                mbar_arrive(b_full + bs.idx);
-              } else {
-                mbar_expect_tx(b_full + bs.idx, kBSlot);
-                bulk_g2s(smem + h.b_off + bs.idx * kBSlot, src, kBSlot, b_full + bs.idx);
-              }
-            }
-            bs.advance(nb);
-          }
-        }
-      }
-      if (dbgp && leader) dbgp[blockIdx.x * 8 + 2] = dbg_b;
-    }
-  } else if (warp == kMmaWarp) {
-    // ===================== MMA issuer =====================
-    // One elected lane issues every tcgen05.mma of the CTA, but ALL 32 lanes run the loop: tcgen05.mma takes
-    // its descriptors from uniform registers, and only values computed in warp-uniform control flow live
-    // there.  With the whole loop inside `if (lane == 0)` the compiler wrapped every MMA in an
-    // ELECT / R2UR.BROADCAST / BRA.U.ANY "waterfall" (~100 cycles per MMA, more than the MMA itself takes).
-    // The per-tap descriptor words come from the kernel parameters (constant bank, uniform index).
-    const bool leader = elect_one_sync();
-    {
-      Ring st, bs;
-      int acc_set = 0;
-      uint32_t acc_phase = 0;
-      long long w_acc = 0, w_a = 0, w_b = 0;
-      const bool timed = dbgp != nullptr;
-      const long long t_start = clock64();
-      const uint32_t plane16 = h.plane_bytes >> 4;
-      const uint32_t lbo_bits = 1u << 16;                 // LBO field (ignored for swizzled K-major; 1 by convention)
-      const uint32_t b_hi_word = (1024u >> 4) | (1u << 14) | (2u << 29);
-      const uint32_t b_base16 = (smem_u32(smem + h.b_off) & 0x3FFFFu) >> 4;
-      constexpr uint32_t kIdescN128 = (1u << 4) | (2u << 7) | (2u << 10) | ((128u >> 3) << 17) | ((128u >> 4) << 24);
-      auto mma = [&](uint32_t d_tmem, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t acc, uint32_t idesc) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-            "mov.b64 da, {%1, %2};\n\t"
-            "mov.b64 db, {%3, %4};\n\t"
-            "setp.ne.b32 p, %6, 0;\n\t"
-            "tcgen05.mma.cta_group::1.kind::tf32 [%0], da, db, %5, p;\n\t}"
-            ::"r"(d_tmem), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi_word), "r"(idesc), "r"(acc)
-            : "memory");
-      };
-      uint32_t cphase = 0;                                // class mode: every set is used once per tile
-      for (int tile = blockIdx.x; tile < h.tiles_total; tile += gridDim.x) {
-        if (ncls == 1) {
-          mbar_wait_timed(acc_empty + acc_set, acc_phase ^ 1, w_acc, timed);   // epilogue has drained this set
-          tc_fence_after();
-        }
-        const uint32_t d0 = tmem_base + acc_set * kAccCols;
-        uint32_t rot = 0;                                 // accumulator block rotation (kb % kRot without a division)
-        int kb = 0;
-        for (int half = 0; half < 2; ++half) {
-          mbar_wait_timed(a_full + st.idx, st.phase, w_a, timed);
-          if (dflags & 128) tc_fence_after();  // not needed: the planes were published with fence.proxy.async
-          const uint32_t stage16 = (smem_u32(smem + st.idx * h.stage_bytes) & 0x3FFFFu) >> 4;
-          for (int t = 0; t < ntaps; ++t, ++kb) {
-            const uint32_t a16 = stage16 + (uint32_t)h.tap_off[t] * 8u;  // slots -> 16-byte units
-            const uint32_t a_hi_word = (((uint32_t)h.tap_hc[t] * 128u) >> 4) | (1u << 14) | (2u << 29);  // SBO, v1, SW128
-            const uint32_t ah = a16 | lbo_bits, al = (a16 + plane16) | lbo_bits;
-            const uint32_t bh = (b_base16 + bs.idx * (kBSlot >> 4)) | lbo_bits;
-            if (!(dflags & 64)) mbar_wait_timed(b_full + bs.idx, bs.phase, w_b, timed);
-            if (dflags & 128) tc_fence_after();  // not needed: bulk-copy (async proxy) data
-            uint32_t d_blk = d0 + rot * kBlkCols;
-            uint32_t acc_first = kb >= kRot;
-            int cls = 0;
-            bool cls_last = false;
-            if (ncls > 1) {
-              cls = h.tap_cls[t];
-              const bool cls_first = t == 0 || h.tap_cls[t - 1] != cls;
-              cls_last = t == ntaps - 1 || h.tap_cls[t + 1] != cls;
-              if (half == 0 && cls_first) {               // the epilogue has drained this class of the previous tile
-                mbar_wait_timed(acc_empty + cls, cphase ^ 1, w_acc, timed);
-                tc_fence_after();
-              }
-              d_blk = tmem_base + cls * kBlkCols;
-              acc_first = !(half == 0 && cls_first);
-            }
-            if (leader) {
-              if (X3) {
-                if (!(dflags & 16)) {
-#pragma unroll
-                  for (int k = 0; k < 4; ++k) mma(d_blk, ah + 2 * k, a_hi_word, bh + 2 * k, k == 0 ? acc_first : 1u, kIdescN128);
-                }
-                if (!(dflags & 24)) {
-#pragma unroll
-                  for (int k = 0; k < 4; ++k) mma(d_blk + 64, al + 2 * k, a_hi_word, bh + 2 * k, 1u, kIdescTf32_128x64);
-                }
-              } else {
-#pragma unroll
-                for (int k = 0; k < 4; ++k) mma(d_blk, ah + 2 * k, a_hi_word, bh + 2 * k, k == 0 ? acc_first : 1u, kIdescTf32_128x64);
-              }
-              if (!(dflags & 32)) umma_commit(b_empty + bs.idx);
-              if (ncls > 1 && half == 1 && cls_last) umma_commit(acc_full + cls);   // class complete
-            }
-            bs.advance(nb);
-            if (ncls == 1 && ++rot == kRot) rot = 0;
-          }
-          if (leader) umma_commit(a_empty + st.idx);
-          st.advance(a_stages);
-        }
-        if (ncls == 1) {
-          if (leader) umma_commit(acc_full + acc_set);
-          if (++acc_set == 2) { acc_set = 0; acc_phase ^= 1; }
-        } else {
-          cphase ^= 1;
-        }
-      }
-      if (timed && leader) {
-        long long* o = dbgp + blockIdx.x * 8;
-        o[3] = w_acc; o[4] = w_a; o[5] = w_b; o[6] = clock64() - t_start;
-      }
-    }
-  } else {
-    halo_epilogue<X3, DBG>(h, acc_full, acc_empty, tmem_base, warp, lane, dflags, dbgp);
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == kWeightWarp) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
-  }
-}
-
-// ------------------------------------------------------------------------------------------------------------
-// TMA-fed variant (default).  Same planes, taps, weight ring, accumulator sets and epilogue; what changes:
-//   warp  14    plane loader: per (tile, channel half) ONE cp.async.bulk.tensor per plane (HaloTma) lands the raw fp32
-//               pixels in the `hi` plane of the stage -- no global-load / address arithmetic in any thread, out-of-bounds
-//               pixels zero-filled by the copy engine;
-//   warps 0-7   split warps: shared memory -> shared memory, one LDS + one STS per 16 bytes (the register-staged
-//               producers spent LDG + address decode + two STS; the L1 data pipe, which the tensor core's operand reads
-//               share, was 95 % busy).  fp32-grade mode: the landed raw plane is used as the `hi` operand as it is -- the
-//               tensor core truncates fp32 to tf32 -- and only lo = x - trunc_tf32(x) is written to the `lo` plane;
-//               single-pass mode: the landed values are rounded to nearest in place;
-//   warp  9     MMA issuer with the tap loop unrolled (NT = 9 or 10 taps): every per-tap descriptor word is a
-//               loop-invariant uniform register, and the `weights landed` probe of tap t+1 is issued before the MMAs of
-//               tap t, so its ~90-cycle latency hides behind the issue of eight MMAs.
-// ------------------------------------------------------------------------------------------------------------
-constexpr int kTmaWarp = kEpiWarp0 + 4;
-constexpr int kThreadsTma = kThreads + 32;
 
 __device__ __forceinline__ float4 lds128(uint32_t saddr) {
   float4 v;
@@ -560,8 +249,8 @@ __device__ __forceinline__ float4 lds128(uint32_t saddr) {
   return v;
 }
 
-template <bool X3, int NT, int NB, bool DBG>
-__global__ void __launch_bounds__(kThreadsTma, 1) tapconv_halo_tma_kernel(const HaloArgs h, const __grid_constant__ HaloTma tm) {
+template <bool X3, int NT, int NB>
+__global__ void __launch_bounds__(kThreads, 1) tapconv_halo_tma_kernel(const HaloArgs h, const __grid_constant__ HaloTma tm) {
   constexpr uint32_t kBSlot = b_slot_bytes<X3>();
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -577,8 +266,6 @@ __global__ void __launch_bounds__(kThreadsTma, 1) tapconv_halo_tma_kernel(const 
   const int nb = h.nb, a_stages = h.a_stages;
 
   const TapConvArgs& a = h.t;
-  const int dflags = DBG ? h.dbg_flags : 0;
-  long long* const dbgp = DBG ? h.dbg : nullptr;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   constexpr uint32_t kAccCols = X3 ? 256u : 128u;
   constexpr uint32_t kTmemCols = 2 * kAccCols;
@@ -587,7 +274,7 @@ __global__ void __launch_bounds__(kThreadsTma, 1) tapconv_halo_tma_kernel(const 
 
   if (tid == 0) {
     for (int s = 0; s < a_stages; ++s) {
-      mbar_init(a_full + s, kProducerThreads);
+      mbar_init(a_full + s, kSplitThreads);
       mbar_init(a_empty + s, 1);
       mbar_init(t_full + s, 1);
     }
@@ -609,7 +296,7 @@ __global__ void __launch_bounds__(kThreadsTma, 1) tapconv_halo_tma_kernel(const 
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
-  if (warp < kProducerWarps) {
+  if (warp < kSplitWarps) {
     // ===================== split warps: smem -> smem =====================
     Ring st;
     const uint32_t units = (uint32_t)h.total_slots * 8u;      // 16-byte units of one plane copy
@@ -617,16 +304,16 @@ __global__ void __launch_bounds__(kThreadsTma, 1) tapconv_halo_tma_kernel(const 
       for (int half = 0; half < 2; ++half) {
         mbar_wait(t_full + st.idx, st.phase);                  // the tensor copies of this stage have landed
         const uint32_t hi = smem_u32(smem + st.idx * h.stage_bytes), lo = hi + h.plane_bytes;
-        for (uint32_t u0 = tid; u0 < units; u0 += 4 * kProducerThreads) {
+        for (uint32_t u0 = tid; u0 < units; u0 += 4 * kSplitThreads) {
           float4 v[4];
 #pragma unroll
           for (int j = 0; j < 4; ++j) {
-            const uint32_t u = u0 + j * kProducerThreads;
+            const uint32_t u = u0 + j * kSplitThreads;
             if (u < units) v[j] = lds128(hi + u * 16u);
           }
 #pragma unroll
           for (int j = 0; j < 4; ++j) {
-            const uint32_t u = u0 + j * kProducerThreads;
+            const uint32_t u = u0 + j * kSplitThreads;
             if (u < units) {
               if (X3) sts128(lo + u * 16u, lo_of_truncated(v[j]));   // the raw plane is the hi operand (hardware truncation)
               else sts128(hi + u * 16u, to_tf32_4(v[j]));            // single pass: round to nearest in place
@@ -658,7 +345,7 @@ __global__ void __launch_bounds__(kThreadsTma, 1) tapconv_halo_tma_kernel(const 
       }
     }
   } else if (warp == kWeightWarp) {
-    // ===================== weight producer =====================
+    // ===================== weight loader =====================
     const bool leader = elect_one_sync();
     Ring bs;
     for (int tile = blockIdx.x; tile < h.tiles_total; tile += gridDim.x)
@@ -676,7 +363,7 @@ __global__ void __launch_bounds__(kThreadsTma, 1) tapconv_halo_tma_kernel(const 
         }
   } else if (warp == kMmaWarp) {
     // ===================== MMA issuer =====================
-    // Work elimination on the register-staged kernel (profiles/halo_stalls_r1.txt) showed MMAs + handshakes alone at
+    // Work elimination on the kernel's first form (profiles/halo_stalls_r1.txt) showed MMAs + handshakes alone at
     // 0.51 of 0.57 ms and the handshake skeleton WITHOUT any MMA at 8.4 K cycles per tile: the issuing lane's own
     // ~100 instructions per K-block (constant-bank loads, R2UR moves, ring arithmetic, a 90-cycle barrier probe) do
     // not overlap the 474 tensor cycles of the K-block, because the tensor queue is shallow.  So here everything that
@@ -798,7 +485,7 @@ __global__ void __launch_bounds__(kThreadsTma, 1) tapconv_halo_tma_kernel(const 
       }
     }
   } else if (warp >= kEpiWarp0 && warp < kEpiWarp0 + 4) {
-    halo_epilogue<X3, DBG>(h, acc_full, acc_empty, tmem_base, warp, lane, dflags, dbgp);
+    halo_epilogue<X3>(h, acc_full, acc_empty, tmem_base, warp, lane);
   }
 
   tc_fence_before();
@@ -808,423 +495,22 @@ __global__ void __launch_bounds__(kThreadsTma, 1) tapconv_halo_tma_kernel(const 
   }
 }
 
-// ------------------------------------------------------------------------------------------------------------
-// 2-SM variant: a CTA PAIR (thread-block cluster of two, one per SM of a TPC) works on two tiles with ONE
-// tcgen05.mma.cta_group::2 stream: M = 256 (128 pixels from each CTA's own planes), the B operand -- the stacked
-// [W_hi ; W_lo] weight K-block -- split along N between the two CTAs.  Per SM that halves the weight-ring fill
-// (8 KB instead of 16 KB per K-block) and the tensor core's B-operand reads, the two largest items of the L1 data
-// pipe budget after the A reads (DESIGN.md finding 17).  Loaders, split warps and epilogue are per CTA and unchanged;
-// the leader CTA's MMA warp issues for the pair, the peer's forwards its barrier completions to the leader
-// (remote mbarrier arrives), and every tcgen05.commit is multicast to the same barrier in both CTAs.
-// ------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// arrive on the barrier at the same shared-memory offset in CTA `target` of the cluster (`issue`: lane predicate)
-__device__ __forceinline__ void remote_arrive(uint64_t* local_bar, uint32_t target, uint32_t issue) {
-  asm volatile(
-      "{\n\t.reg .pred q;\n\t.reg .b32 ra;\n\t"
-      "setp.ne.b32 q, %2, 0;\n\t"
-      "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-      "@q mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t}"
-      ::"r"(smem_u32(local_bar)), "r"(target), "r"(issue)
-      : "memory");
-}
-// wait for an arrival that came from the peer CTA.  Plain CTA-scope wait, as CUTLASS's ClusterBarrier does: what the
-// arrival orders is read by the PEER's tensor core from the peer's own shared memory, not by this CTA's threads (a
-// cluster-scope acquire here costs an L1 invalidation per wait: the first version of this kernel ran at half speed)
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-  uint32_t spins = 0;
-  uint64_t t0 = 0;
-  for (;;) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    if (ok) return;
-    if ((++spins & 0xffffu) == 0) {
-      uint64_t t;
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-      if (t0 == 0) t0 = t;
-      else if (t - t0 > 20000000000ull) __trap();
-    }
-  }
-}
-
-template <bool X3, int NT, int NB, bool DBG>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsTma, 1) tapconv_halo_tma2_kernel(const HaloArgs h, const __grid_constant__ HaloTma tm) {
-  constexpr uint32_t kBSlot = b_slot_bytes<X3>();
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + h.bar_off);
-  uint64_t* a_full = bars;                  // [a_stages] split warps -> MMA          (count 256)
-  uint64_t* a_empty = bars + 2;             // [a_stages] MMA commit -> plane loader  (count 1)
-  uint64_t* acc_full = bars + 4;            // [4] MMA commit -> epilogue             (count 1)
-  uint64_t* acc_empty = bars + 8;           // [4] epilogue -> MMA                    (count 128)
-  uint64_t* b_full = bars + 12;             // [nb] bulk copy tx -> MMA               (count 1 + tx)
-  uint64_t* b_empty = b_full + kMaxBStages; // [nb] MMA commit -> weight warp         (count 1)
-  uint64_t* t_full = b_empty + kMaxBStages; // [a_stages] tensor copies tx -> split warps, MMA (count 1 + tx)
-  uint64_t* p_afull = t_full + 2;           // leader only, [a_stages]: the PEER's stage is ready        (count 1, relayed)
-  uint64_t* p_accempty = p_afull + 2;       // leader only, [4]: the PEER's epilogue has drained the set     (count 1, relayed)
-  uint64_t* p_bfull = p_accempty + 4;       // leader only, [nb]: the PEER's half of the weight slot landed (count 1, relayed)
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(p_bfull + kMaxBStages);
-  const int nb = h.nb, a_stages = h.a_stages;
-  uint32_t cta_rank;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(cta_rank));
-
-  const TapConvArgs& a = h.t;
-  const int dflags = DBG ? h.dbg_flags : 0;
-  long long* const dbgp = DBG ? h.dbg : nullptr;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  constexpr uint32_t kAccCols = X3 ? 256u : 128u;
-  constexpr uint32_t kTmemCols = 2 * kAccCols;
-  constexpr uint32_t kBlkCols = X3 ? 128u : 64u;
-  const int ncls = h.ncls;
-
-  if (tid == 0) {
-    for (int s = 0; s < a_stages; ++s) {
-      mbar_init(a_full + s, kProducerThreads);
-      mbar_init(a_empty + s, 1);
-      mbar_init(t_full + s, 1);
-    }
-    for (int s = 0; s < nb; ++s) { mbar_init(b_full + s, 1); mbar_init(b_empty + s, 1); }
-    for (int s = 0; s < 4; ++s) { mbar_init(acc_full + s, 1); mbar_init(acc_empty + s, 128); mbar_init(p_accempty + s, 1); }
-    for (int s = 0; s < 2; ++s) mbar_init(p_afull + s, 1);
-    for (int s = 0; s < nb; ++s) mbar_init(p_bfull + s, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == kWeightWarp) {
-    // one warp of EACH CTA of the pair, same warp index, same destination offset (cute::TMEM::Allocator2Sm)
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(kTmemCols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  if (warp == kTmaWarp && lane == 0) {
-    for (int p = 0; p < h.nplanes; ++p) tma::prefetch_map(&tm.plane[p]);
-  }
-  tc_fence_before();
-  cluster_sync_all();        // both CTAs' barriers are initialised before any remote arrive / multicast commit
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp < kProducerWarps) {
-    // ===================== split warps: smem -> smem =====================
-    Ring st;
-    const uint32_t units = (uint32_t)h.total_slots * 8u;      // 16-byte units of one plane copy
-    for (int tile = blockIdx.x; tile < h.tiles_total; tile += gridDim.x)
-      for (int half = 0; half < 2; ++half) {
-        mbar_wait(t_full + st.idx, st.phase);                  // the tensor copies of this stage have landed
-        const uint32_t hi = smem_u32(smem + st.idx * h.stage_bytes), lo = hi + h.plane_bytes;
-        for (uint32_t u0 = tid; u0 < units; u0 += 4 * kProducerThreads) {
-          float4 v[4];
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const uint32_t u = u0 + j * kProducerThreads;
-            if (u < units) v[j] = lds128(hi + u * 16u);
-          }
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const uint32_t u = u0 + j * kProducerThreads;
-            if (u < units) {
-              if (X3) sts128(lo + u * 16u, lo_of_truncated(v[j]));   // the raw plane is the hi operand (hardware truncation)
-              else sts128(hi + u * 16u, to_tf32_4(v[j]));            // single pass: round to nearest in place
-            }
-          }
-        }
-        fence_proxy_async();
-        mbar_arrive(a_full + st.idx);
-        st.advance(a_stages);
-      }
-  } else if (warp == kTmaWarp) {
-    // ===================== plane loader (TMA) =====================
-    const uint32_t leader = elect_one_sync();
-    Ring st;
-    uint32_t stage_tx = 0;
-    for (int p = 0; p < h.nplanes; ++p) stage_tx += (uint32_t)(h.pl[p].HR * h.pl[p].HC) * 128u;
-    for (int tile = blockIdx.x; tile < h.tiles_total; tile += gridDim.x) {
-      const int xt = tile % h.tiles_x, rb = tile / h.tiles_x;
-      const int r0 = rb * kTileRows;
-      const int n = r0 / a.OH, oy0 = r0 - n * a.OH, ox0 = xt * kTileCols;
-      for (int half = 0; half < 2; ++half) {
-        mbar_wait(a_empty + st.idx, st.phase ^ 1);             // the MMAs that read this stage have retired
-        if (leader) mbar_expect_tx(t_full + st.idx, stage_tx);
-        const uint32_t stage = smem_u32(smem + st.idx * h.stage_bytes);
-        for (int p = 0; p < h.nplanes; ++p)
-          tma::load_4d(stage + (uint32_t)h.pl[p].slot0 * 128u, &tm.plane[p], smem_u32(t_full + st.idx), half * 32,
-                       ox0 + h.pl[p].dx_min, oy0 + h.pl[p].dy_min, n, leader);
-        st.advance(a_stages);
-      }
-    }
-  } else if (warp == kWeightWarp) {
-    // ===================== weight producer =====================
-    const bool leader = elect_one_sync();
-    Ring bs;
-    for (int tile = blockIdx.x; tile < h.tiles_total; tile += gridDim.x)
-      for (int half = 0; half < 2; ++half)
-#pragma unroll
-        for (int t = 0; t < NT; ++t) {
-          const Tap tp = a.taps[t];
-          // this CTA's half of the B operand: fp32-grade  rank 0 = W_hi (rows 0-63 of [W_hi ; W_lo]), rank 1 = W_lo;
-          // single pass  rows 32 r .. 32 r + 31 of W_hi (K-major SWIZZLE_128B tile: 1024 B per 8 rows)
-          const float* src = h.bp[tp.src] + ((long long)half * h.nslabs[tp.src] + tp.slab) * (kBSlotBytes / 4) +
-                             cta_rank * (kBSlot / 8);
-          mbar_wait(b_empty + bs.idx, bs.phase ^ 1);
-          if (leader) {
-            mbar_expect_tx(b_full + bs.idx, kBSlot / 2);
-            bulk_g2s(smem + h.b_off + bs.idx * kBSlot, src, kBSlot / 2, b_full + bs.idx);
-          }
-          bs.advance(nb);
-        }
-  } else if (warp == kMmaWarp && cta_rank != 0 && (h.dbg_flags & 256)) {
-    // diagnostics: no relay (results undefined)
-  } else if (warp == kMmaWarp && cta_rank != 0) {
-    // ===================== peer CTA: relay =====================
-    // The leader issues the pair's MMAs, so it must know when THIS CTA's operands and accumulators are ready.  This
-    // warp waits on the local barriers in exactly the order the leader consumes them and forwards each completion to
-    // the leader's p_* barrier of the same index (remote mbarrier arrive, cluster scope).
-    static_assert((2 * NT) % NB == 0, "ring depth must divide the K-blocks of a tile");
-    constexpr uint32_t kWraps = 2 * NT / NB;
-    const uint32_t leader = elect_one_sync();
-    int acc_set = 0;
-    uint32_t acc_phase = 0, cphase = 0, it = 0;
-    for (int tile = blockIdx.x; tile < h.tiles_total; tile += gridDim.x, ++it) {
-      if (ncls == 1) {
-        mbar_wait(acc_empty + acc_set, acc_phase ^ 1);
-        remote_arrive(p_accempty + acc_set, 0, leader);
-      }
-      const uint32_t ring_par0 = it * kWraps;
-#pragma unroll
-      for (int half = 0; half < 2; ++half) {
-        const uint32_t sidx = a_stages == 2 ? (uint32_t)half : 0u;
-        const uint32_t spar = a_stages == 2 ? (it & 1u) : ((2u * it + half) & 1u);
-        mbar_wait(t_full + sidx, spar);
-        mbar_wait(a_full + sidx, spar);
-        remote_arrive(p_afull + sidx, 0, leader);
-#pragma unroll
-        for (int t = 0; t < NT; ++t) {
-          const int kb = half * NT + t;
-          const uint32_t slot = (uint32_t)(kb % NB), pass = (uint32_t)(kb / NB);
-          if (ncls > 1) {
-            const int cls = h.tap_cls[t];
-            const bool cls_first = t == 0 || h.tap_cls[t > 0 ? t - 1 : 0] != cls;
-            if (half == 0 && cls_first) {
-              mbar_wait(acc_empty + cls, cphase ^ 1);
-              remote_arrive(p_accempty + cls, 0, leader);
-            }
-          }
-          mbar_wait(b_full + slot, (ring_par0 + pass) & 1u);
-          remote_arrive(p_bfull + slot, 0, leader);
-        }
-      }
-      if (ncls == 1) {
-        if (++acc_set == 2) { acc_set = 0; acc_phase ^= 1; }
-      } else {
-        cphase ^= 1;
-      }
-    }
-  } else if (warp == kMmaWarp) {
-    // ===================== leader CTA: MMA issuer for the pair (tcgen05.mma.cta_group::2) =====================
-    // M = 256: rows 0-127 are the leader's tile, rows 128-255 the peer's (each from its own shared memory, same
-    // descriptor); N = 128 = [W_hi ; W_lo], rows 0-63 in the leader's weight slot, 64-127 in the peer's: each CTA fills
-    // and its tensor core reads HALF of every weight K-block.  fp32-grade: A_hi x [W_hi ; W_lo] and A_lo x [W_hi ; W_lo]
-    // into the SAME 128 columns (columns 0-63 collect hi*hi + lo*hi, 64-127 hi*lo + lo*lo; the epilogue adds the halves
-    // as before) -- both instructions take the same B descriptor, which is what lets the N split work for both.
-    static_assert((2 * NT) % NB == 0, "ring depth must divide the K-blocks of a tile");
-    constexpr uint32_t kWraps = 2 * NT / NB;
-    const uint32_t leader = elect_one_sync();
-    int acc_set = 0;
-    uint32_t acc_phase = 0, cphase = 0;
-    const uint32_t plane16 = h.plane_bytes >> 4;
-    const uint32_t lbo_bits = 1u << 16;
-    const uint32_t b_hi_word = (1024u >> 4) | (1u << 14) | (2u << 29);
-    const uint32_t b_base16 = ((smem_u32(smem + h.b_off) & 0x3FFFFu) >> 4) | lbo_bits;
-    const uint32_t smem16 = (smem_u32(smem) & 0x3FFFFu) >> 4;
-    const uint32_t stage16_step = h.stage_bytes >> 4;
-    const uint32_t b_full_a = smem_u32(b_full), b_empty_a = smem_u32(b_empty);
-    constexpr uint32_t kIdesc2 = (1u << 4) | (2u << 7) | (2u << 10) | (((X3 ? 128u : 64u) >> 3) << 17) | ((256u >> 4) << 24);
-    uint32_t a_off16[NT], a_hiw[NT];
-#pragma unroll
-    for (int t = 0; t < NT; ++t) {
-      a_off16[t] = (uint32_t)h.tap_off[t] * 8u;
-      a_hiw[t] = (((uint32_t)h.tap_hc[t] * 128u) >> 4) | (1u << 14) | (2u << 29);
-    }
-    auto mma = [&](uint32_t d_tmem, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t acc) {
-      asm volatile(
-          "{\n\t.reg .pred p, q;\n\t.reg .b64 da, db;\n\t"
-          "mov.b64 da, {%1, %2};\n\t"
-          "mov.b64 db, {%3, %4};\n\t"
-          "setp.ne.b32 p, %6, 0;\n\t"
-          "setp.ne.b32 q, %7, 0;\n\t"
-          "@q tcgen05.mma.cta_group::2.kind::tf32 [%0], da, db, %5, p;\n\t}"
-          ::"r"(d_tmem), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi_word), "r"(kIdesc2), "r"(acc), "r"(leader)
-          : "memory");
-    };
-    auto commit2 = [&](uint32_t bar_addr) {   // arrives on the barrier at this offset in BOTH CTAs
-      asm volatile(
-          "{\n\t.reg .pred q;\n\t.reg .b16 m;\n\t"
-          "setp.ne.b32 q, %1, 0;\n\t"
-          "mov.b16 m, 3;\n\t"
-          "@q tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], m;\n\t}"
-          ::"r"(bar_addr), "r"(leader)
-          : "memory");
-    };
-    auto probe = [&](uint32_t bar_addr, uint32_t parity) -> bool {
-      uint32_t ok;
-      asm volatile(
-          "{\n\t.reg .pred p;\n\t"
-          "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-          "selp.u32 %0, 1, 0, p;\n\t}"
-          : "=r"(ok)
-          : "r"(bar_addr), "r"(parity)
-          : "memory");
-      return ok != 0;
-    };
-    bool b_ready = false;
-    const bool norelay = (h.dbg_flags & 256) != 0;           // diagnostics: do not wait for the peer (results undefined)
-    uint32_t it = 0;
-    for (int tile = blockIdx.x; tile < h.tiles_total; tile += gridDim.x, ++it) {
-      if (ncls == 1) {
-        mbar_wait(acc_empty + acc_set, acc_phase ^ 1);       // own epilogue has drained this set ...
-        if (!norelay) mbar_wait_cluster(p_accempty + acc_set, acc_phase);  // ... and so has the peer's
-        tc_fence_after();
-      }
-      const uint32_t d0 = tmem_base + acc_set * kAccCols;
-      const uint32_t ring_par0 = it * kWraps;
-#pragma unroll
-      for (int half = 0; half < 2; ++half) {
-        const uint32_t sidx = a_stages == 2 ? (uint32_t)half : 0u;
-        const uint32_t spar = a_stages == 2 ? (it & 1u) : ((2u * it + half) & 1u);
-        mbar_wait(t_full + sidx, spar);
-        mbar_wait(a_full + sidx, spar);
-        if (!norelay) mbar_wait_cluster(p_afull + sidx, spar);
-        const uint32_t stage16 = (smem16 + sidx * stage16_step) | lbo_bits;
-#pragma unroll
-        for (int t = 0; t < NT; ++t) {
-          const int kb = half * NT + t;
-          const uint32_t slot = (uint32_t)(kb % NB), pass = (uint32_t)(kb / NB);
-          const uint32_t kbn = (uint32_t)((kb + 1) % (2 * NT));
-          const uint32_t slot_n = kbn % NB, pass_n = kbn / NB + (kb + 1 == 2 * NT ? kWraps : 0u);
-          uint32_t d_blk = d0 + (uint32_t)(kb % kRot) * kBlkCols;
-          uint32_t acc_first = kb >= kRot;
-          int cls = 0;
-          bool cls_last = false;
-          if (ncls > 1) {
-            cls = h.tap_cls[t];
-            const bool cls_first = t == 0 || h.tap_cls[t > 0 ? t - 1 : 0] != cls;
-            cls_last = t == NT - 1 || h.tap_cls[t < NT - 1 ? t + 1 : t] != cls;
-            if (half == 0 && cls_first) {
-              mbar_wait(acc_empty + cls, cphase ^ 1);
-              if (!norelay) mbar_wait_cluster(p_accempty + cls, cphase);
-              tc_fence_after();
-            }
-            d_blk = tmem_base + cls * kBlkCols;
-            acc_first = !(half == 0 && cls_first);
-          }
-          if (!b_ready) {
-            mbar_wait(b_full + slot, (ring_par0 + pass) & 1u);
-            if (!norelay) mbar_wait_cluster(p_bfull + slot, (ring_par0 + pass) & 1u);
-          }
-          {   // probe the NEXT slot in both CTAs now, use the answer after these MMAs
-            const bool own = probe(b_full_a + slot_n * 8u, (ring_par0 + pass_n) & 1u);
-            const bool peer = norelay || probe(smem_u32(p_bfull) + slot_n * 8u, (ring_par0 + pass_n) & 1u);
-            b_ready = own && peer;
-          }
-          const uint32_t ah = stage16 + a_off16[t], al = ah + plane16;
-          const uint32_t bh = b_base16 + slot * (kBSlot >> 4);
-#pragma unroll
-          for (int k = 0; k < 4; ++k) mma(d_blk, ah + 2 * k, a_hiw[t], bh + 2 * k, k == 0 ? acc_first : 1u);
-          if (X3 && !(h.dbg_flags & 512)) {
-#pragma unroll
-            for (int k = 0; k < 4; ++k) mma(d_blk, al + 2 * k, a_hiw[t], bh + 2 * k, 1u);
-          }
-          commit2(b_empty_a + slot * 8u);
-          if (ncls > 1 && half == 1 && cls_last) commit2(smem_u32(acc_full + cls));
-        }
-        commit2(smem_u32(a_empty + sidx));
-      }
-      if (ncls == 1) {
-        commit2(smem_u32(acc_full + acc_set));
-        if (++acc_set == 2) { acc_set = 0; acc_phase ^= 1; }
-      } else {
-        cphase ^= 1;
-      }
-    }
-  } else if (warp >= kEpiWarp0 && warp < kEpiWarp0 + 4) {
-    halo_epilogue<X3, DBG>(h, acc_full, acc_empty, tmem_base, warp, lane, dflags, dbgp);
-  }
-
-  tc_fence_before();
-  cluster_sync_all();        // the pair's MMAs and multicast commits touch both CTAs: leave together
-  if (warp == kWeightWarp) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
-  }
-}
-
-template <bool X3, int NT, int NB>
-int launch_halo_tma2_t(const HaloArgs& h, const HaloTma& tm, size_t smem, cudaStream_t st) {
-  static size_t configured = 0;
-  if (smem > configured) {
-    if (cudaFuncSetAttribute(tapconv_halo_tma2_kernel<X3, NT, NB, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)smem) != cudaSuccess)
-      return B200NP_E_LAUNCH;
-    configured = smem;
-  }
-  int grid = (h.tiles_total < kNumSMs ? h.tiles_total : kNumSMs) & ~1;   // whole CTA pairs
-  tapconv_halo_tma2_kernel<X3, NT, NB, false><<<grid, kThreadsTma, smem, st>>>(h, tm);
-  return launch_status();
-}
-
 template <bool X3, int NT, int NB>
 int launch_halo_tma_t(const HaloArgs& h, const HaloTma& tm, size_t smem, cudaStream_t st) {
   static size_t configured = 0;
   if (smem > configured) {
-    if (cudaFuncSetAttribute(tapconv_halo_tma_kernel<X3, NT, NB, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    if (cudaFuncSetAttribute(tapconv_halo_tma_kernel<X3, NT, NB>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)smem) != cudaSuccess)
       return B200NP_E_LAUNCH;
     configured = smem;
   }
   int grid = h.tiles_total < kNumSMs ? h.tiles_total : kNumSMs;
-  tapconv_halo_tma_kernel<X3, NT, NB, false><<<grid, kThreadsTma, smem, st>>>(h, tm);
+  tapconv_halo_tma_kernel<X3, NT, NB><<<grid, kThreads, smem, st>>>(h, tm);
   return launch_status();
-}
-
-template <bool X3, int MAXT>
-int launch_halo_t(const HaloArgs& h, size_t smem, cudaStream_t st) {
-  static size_t configured = 0;
-  if (smem > configured) {
-    if (cudaFuncSetAttribute(tapconv_halo_kernel<X3, MAXT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)smem) != cudaSuccess ||
-        cudaFuncSetAttribute(tapconv_halo_kernel<X3, MAXT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)smem) != cudaSuccess)
-      return B200NP_E_LAUNCH;
-    configured = smem;
-  }
-  int grid = h.tiles_total < kNumSMs ? h.tiles_total : kNumSMs;
-  if (h.dbg || h.dbg_flags) tapconv_halo_kernel<X3, MAXT, true><<<grid, kThreads, smem, st>>>(h);
-  else tapconv_halo_kernel<X3, MAXT, false><<<grid, kThreads, smem, st>>>(h);
-  return launch_status();
-}
-
-// B200NP_HALO_TMA=0 keeps the register-staged kernel (the TMA-fed one is the default where its tensor maps can be built)
-static bool halo_tma_enabled() {
-  static const bool on = [] { const char* e = getenv("B200NP_HALO_TMA"); return e ? e[0] != '0' : true; }();
-  return on;
-}
-
-// B200NP_HALO_CG2=1 selects the 2-SM (cta_group::2) form of the TMA-fed kernel
-static bool halo_cg2_enabled() {
-  static const bool on = [] { const char* e = getenv("B200NP_HALO_CG2"); return (e && e[0]) ? e[0] != '0' : false; }();
-  return on;
 }
 
 // One tensor map per plane (see HaloTma).  false: some plane cannot be expressed (odd extent under a stride-2 view,
-// driver without tensor-map support) -- the caller falls back to the register-staged kernel.
+// driver without tensor-map support) -- the convolution then runs on the gather kernel.
 static bool build_plane_maps(const HaloArgs& h, HaloTma& tm) {
   for (int p = 0; p < h.nplanes; ++p) {
     const Plane& P = h.pl[p];
@@ -1248,7 +534,8 @@ static bool build_plane_maps(const HaloArgs& h, HaloTma& tm) {
 
 template <bool X3>
 int launch_halo(HaloArgs& h, cudaStream_t st) {
-  // shared-memory plan: one or two plane stages, then as deep a weight ring as fits (>= 2 slots)
+  // shared-memory plan: one or two plane stages, then a weight ring whose depth divides the 2 * ntaps K-blocks of a
+  // tile (the MMA issuer's slot indices are compile-time constants): 4 slots for 10 taps, 6 or 3 for 9
   const uint32_t planes = X3 ? 2u : 1u;
   h.plane_bytes = (uint32_t)h.total_slots * 128u;
   h.stage_bytes = planes * h.plane_bytes;
@@ -1257,31 +544,15 @@ int launch_halo(HaloArgs& h, cudaStream_t st) {
   h.a_stages = (2 * h.stage_bytes + 2 * bslot + tail <= kSmemBudget) ? 2 : 1;
   if (h.a_stages * h.stage_bytes + 2 * bslot + tail > kSmemBudget) return B200NP_E_UNSUPPORTED;
   h.b_off = h.a_stages * h.stage_bytes;
-  int nb = (int)((kSmemBudget - tail - h.b_off) / bslot);
-  if (nb > kMaxBStages) nb = kMaxBStages;
-  h.nb = nb;
-  h.bar_off = h.b_off + nb * bslot;
+  const int nb = (int)((kSmemBudget - tail - h.b_off) / bslot);
+  const int want = h.t.ntaps == 10 ? 4 : (nb >= 6 ? 6 : 3);
+  HaloTma tm;
+  if (nb < want || !build_plane_maps(h, tm)) return B200NP_E_UNSUPPORTED;
+  h.nb = want;
+  h.bar_off = h.b_off + want * bslot;
   const size_t smem = h.bar_off + tail;
-  const int tasks = (h.total_slots + kSlotsPerPass - 1) / kSlotsPerPass;
-  if (halo_tma_enabled() && !h.dbg && !(h.dbg_flags & 255) && (h.t.ntaps == 9 || h.t.ntaps == 10)) {
-    // the TMA-fed kernel wants a weight ring whose depth divides the 2 * ntaps K-blocks of a tile (compile-time slots)
-    const int want = h.t.ntaps == 10 ? 4 : (nb >= 6 ? 6 : 3);
-    HaloTma tm;
-    if (nb >= want && build_plane_maps(h, tm)) {
-      h.nb = want;
-      h.bar_off = h.b_off + want * bslot;
-      const size_t smem_t = h.bar_off + tail;
-      if (halo_cg2_enabled() && h.tiles_total >= 2 && !(h.tiles_total & 1)) {   // CTA pairs (2-SM MMA)
-        if (h.t.ntaps == 10) return launch_halo_tma2_t<X3, 10, 4>(h, tm, smem_t, st);
-        return want == 6 ? launch_halo_tma2_t<X3, 9, 6>(h, tm, smem_t, st) : launch_halo_tma2_t<X3, 9, 3>(h, tm, smem_t, st);
-      }
-      if (h.t.ntaps == 10) return launch_halo_tma_t<X3, 10, 4>(h, tm, smem_t, st);
-      return want == 6 ? launch_halo_tma_t<X3, 9, 6>(h, tm, smem_t, st) : launch_halo_tma_t<X3, 9, 3>(h, tm, smem_t, st);
-    }
-  }
-  if (tasks <= 10) return launch_halo_t<X3, 10>(h, smem, st);
-  if (tasks <= 18) return launch_halo_t<X3, 18>(h, smem, st);
-  return B200NP_E_UNSUPPORTED;
+  if (h.t.ntaps == 10) return launch_halo_tma_t<X3, 10, 4>(h, tm, smem, st);
+  return want == 6 ? launch_halo_tma_t<X3, 9, 6>(h, tm, smem, st) : launch_halo_tma_t<X3, 9, 3>(h, tm, smem, st);
 }
 
 }  // namespace
@@ -1289,11 +560,11 @@ int launch_halo(HaloArgs& h, cudaStream_t st) {
 // Eligibility + geometry.  `bp0` / `bp1`: pre-split weights of source 0 / 1 (see b200np_pack_conv_weight).
 int launch_tapconv_halo(const TapConvArgs& a, const float* bp0, int nslabs0, const float* bp1, int nslabs1,
                         int precision, cudaStream_t st, const TapClasses* cls) {
-  if (a.Cin != 64 || a.Cout != 64 || a.ntaps < 1 || a.ntaps > kMaxTaps || !bp0) return B200NP_E_UNSUPPORTED;
+  // the MMA issuer unrolls the tap loop: 9 taps (3x3), or 10 (3x3 + the fused 1x1 skip)
+  if (a.Cin != 64 || a.Cout != 64 || (a.ntaps != 9 && a.ntaps != 10) || !bp0) return B200NP_E_UNSUPPORTED;
   if (a.act != B200NP_ACT_NONE && a.act != B200NP_ACT_RELU) return B200NP_E_UNSUPPORTED;
   if (a.OH % kTileRows != 0 || a.OW % kTileCols != 0) return B200NP_E_UNSUPPORTED;
   if (a.in_s[0] != 1 && a.in_s[0] != 2) return B200NP_E_UNSUPPORTED;
-  if (a.ntaps < g_halo_min_taps) return B200NP_E_UNSUPPORTED;
   HaloArgs h{};
   h.t = a;
   h.ncls = 1;
@@ -1312,8 +583,6 @@ int launch_tapconv_halo(const TapConvArgs& a, const float* bp0, int nslabs0, con
       if (!any) return B200NP_E_UNSUPPORTED;
     }
   }
-  h.dbg = g_halo_dbg;
-  h.dbg_flags = g_halo_flags;
   h.bp[0] = bp0; h.bp[1] = bp1; h.nslabs[0] = nslabs0; h.nslabs[1] = nslabs1;
   // group the taps into planes: (source, row parity, column parity) for a stride-2 source, one plane otherwise
   struct Key { int src, py, px; } keys[kMaxPlanes];

@@ -20,7 +20,17 @@
 // kernel's, so the same reduction follows.  Role 0 also sums dY for the bias gradient.
 // Measured as a prototype (tools/probe/wgrad_halo_proto.cu, 12 tap-products): 0.69 ms against 0.80 ms for the 9 taps +
 // reduction of the gather kernel at 1140 images.
-#include <cstdlib>
+//
+// Warp-specialised CTA; full/empty mbarriers hand two stages over, so the tensor core works on tile i while the loader
+// and the split warps prepare tile i+1:
+//   warp 8      loader: per tile one cp.async.bulk.tensor per (row, 32-channel block) of the x halo, the skip rows and
+//               the dY tile drops the raw fp32 pixels into the `hi` regions of a stage (4-D maps [channel][x][y][image],
+//               box 32 x pixels x 1 x 1, SWIZZLE_128B_ATOM_32B = the MN-major operand swizzle; image borders arrive as
+//               zeros) -- no global load, no address arithmetic in any thread;
+//   warps 0-7   split warps, shared memory -> shared memory (split_sweep): the tf32 hi / lo operands and the dY column
+//               sums for the bias gradient;
+//   warp 9      MMA issuer only.  (A block-synchronous form, in which warp 0 issued a tile's 48 MMAs and then helped
+//               stage the next one, paid T_tile = T_issue + T_store: 0.79 ms against 0.56 ms.)
 
 #include "tapconv.cuh"
 #include "tma.cuh"
@@ -39,10 +49,6 @@ constexpr uint32_t A1_PLANE = RT * 4 * S_A;              // role 1: [row][x cb0 
 constexpr uint32_t S_B = TW * 128;                       // one channel block of one dY row: 2048 B
 constexpr uint32_t B_TILE = RT * 4 * S_B;                // [row][hi | lo][block][pixel]
 constexpr uint32_t STAGE = 2 * A1_PLANE + B_TILE;        // sized for role 1 (the larger): 106496 B = 104 * 1024
-constexpr int kThreads = 256;
-constexpr int XT0 = ((RT + 1) * HW * 16 + kThreads - 1) / kThreads;   // 16-byte tasks per thread: role 0 x halo (6)
-constexpr int XT1 = (RT * (HW + TW) * 16 + kThreads - 1) / kThreads;  // role 1: x rows + skip rows (9)
-constexpr int YT = RT * TW * 16 / kThreads;                           // dY tile (4)
 constexpr uint32_t kIdesc128x64 = kIdescTf32_128x64 | (1u << 15) | (1u << 16);
 constexpr uint32_t kIdesc128x128 =
     (1u << 4) | (2u << 7) | (2u << 10) | (1u << 15) | (1u << 16) | ((128u >> 3) << 17) | ((128u >> 4) << 24);
@@ -56,7 +62,6 @@ struct HaloWgradArgs {
   float* part_db;      // nullable: [chunks][64]
   int N, H, W, ntaps;  // ntaps = 9 or 10 (with skip)
   long long tiles, per;
-  int only_role;       // diagnostics (B200NP_WGRAD_ONLY_ROLE=0|1: time one role alone, results incomplete); -1 = both
 };
 
 __device__ __forceinline__ uint64_t mn_desc(uint32_t saddr, uint32_t lbo) {
@@ -68,209 +73,13 @@ __device__ __forceinline__ uint64_t mn_desc(uint32_t saddr, uint32_t lbo) {
   d |= static_cast<uint64_t>(1) << 61;          // SWIZZLE_128B_BASE32B, base_offset 0
   return d;
 }
-// byte offset of 16-byte chunk `chunk` (0..7) inside the 128-byte row at byte offset `row` of a region whose base is a
-// multiple of 512 B from a 1024-aligned stage
-__device__ __forceinline__ uint32_t swz(uint32_t row, int chunk) {
-  return row + ((((chunk >> 1) ^ ((row >> 7) & 3)) << 5) | ((chunk & 1) << 4));
-}
 
-template <bool X3, int ROLE>
-__device__ __forceinline__ void run_role(const HaloWgradArgs& a, uint8_t* smem, uint64_t* bars, uint32_t tmem) {
-  constexpr int XT = ROLE == 0 ? XT0 : XT1;
-  constexpr uint32_t A_PLANE = ROLE == 0 ? A0_PLANE : A1_PLANE;
-  constexpr uint32_t ROW_A = ROLE == 0 ? 2 * S_A : 4 * S_A;   // distance between the first halves of consecutive rows
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int warp_u = __shfl_sync(0xffffffffu, warp, 0);
-  const uint32_t leader = elect_one_sync();
-  const int chunk = blockIdx.x;
-  const int H = a.H, W = a.W;
-  const int tiles_x = W / TW, tiles_img = tiles_x * (H / RT);
-  const long long t_begin = chunk * a.per, t_end = t_begin + a.per < a.tiles ? t_begin + a.per : a.tiles;
-  const int c16 = tid & 15;                      // this thread's 16-byte chunk of a pixel (the same for all its tasks)
-
-  float4 xv[XT], yv[YT];
-  float4 dbs = make_float4(0.f, 0.f, 0.f, 0.f);
-  auto fetch = [&](long long tile) {
-    const int n = (int)(tile / tiles_img), rem = (int)(tile - (long long)n * tiles_img);
-    const int oy0 = (rem / tiles_x) * RT, ox0 = (rem % tiles_x) * TW;
-#pragma unroll
-    for (int i = 0; i < XT; ++i) {
-      const int px = (tid + i * kThreads) >> 4;
-      xv[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (ROLE == 0) {          // x halo: row hr <-> image row oy0 + hr - 1, column pc <-> ox0 + pc - 1
-        const int hr = px / HW, pc = px - hr * HW;
-        const int iy = oy0 + hr - 1, ix = ox0 + pc - 1;
-        if (px < (RT + 1) * HW && (unsigned)iy < (unsigned)H && (unsigned)ix < (unsigned)W)
-          xv[i] = ldg4(a.x + (((long long)n * H + iy) * W + ix) * 64 + c16 * 4);
-      } else if (px < RT * HW) {   // x rows for dy = +1: row r <-> image row oy0 + r + 1
-        const int r = px / HW, pc = px - r * HW;
-        const int iy = oy0 + r + 1, ix = ox0 + pc - 1;
-        if ((unsigned)iy < (unsigned)H && (unsigned)ix < (unsigned)W)
-          xv[i] = ldg4(a.x + (((long long)n * H + iy) * W + ix) * 64 + c16 * 4);
-      } else if (px < RT * (HW + TW)) {   // skip rows: pixel k of row r <-> xs[2 (oy0 + r)][2 (ox0 + k)]
-        const int q = px - RT * HW, r = q / TW, k = q - r * TW;
-        if (a.xs) xv[i] = ldg4(a.xs + (((long long)n * 2 * H + 2 * (oy0 + r)) * 2 * W + 2 * (ox0 + k)) * 64 + c16 * 4);
-      }
-    }
-#pragma unroll
-    for (int i = 0; i < YT; ++i) {
-      const int px = (tid + i * kThreads) >> 4;
-      const int r = px / TW, pc = px - r * TW;
-      yv[i] = ldg4(a.dy + (((long long)n * H + oy0 + r) * W + ox0 + pc) * 64 + c16 * 4);
-    }
-  };
-  auto store = [&](uint8_t* st) {
-    uint8_t* a_hi = st;
-    uint8_t* a_lo = st + A_PLANE;
-    uint8_t* b = st + 2 * A_PLANE;
-    const int cb = c16 >> 3, ch = c16 & 7;
-#pragma unroll
-    for (int i = 0; i < XT; ++i) {
-      const int px = (tid + i * kThreads) >> 4;
-      if (ROLE == 0) {
-        const int hr = px / HW, pc = px - hr * HW;
-        if (px < (RT + 1) * HW) split_store(a_hi, a_lo, swz((uint32_t)(hr * 2 + cb) * S_A + pc * 128, ch), xv[i], X3);
-      } else if (px < RT * HW) {
-        const int r = px / HW, pc = px - r * HW;
-        split_store(a_hi, a_lo, swz((uint32_t)(r * 4 + cb) * S_A + pc * 128, ch), xv[i], X3);
-      } else if (px < RT * (HW + TW)) {   // skip pixel k sits at column k + 1: the dx = 0 pair (start column 1) reads it
-        const int q = px - RT * HW, r = q / TW, k = q - r * TW;
-        split_store(a_hi, a_lo, swz((uint32_t)(r * 4 + 2 + cb) * S_A + (k + 1) * 128, ch), xv[i], X3);
-      }
-    }
-#pragma unroll
-    for (int i = 0; i < YT; ++i) {
-      const int px = (tid + i * kThreads) >> 4;
-      const int r = px / TW, pc = px - r * TW;
-      split_store(b, b + 2 * S_B, swz((uint32_t)(r * 4 + cb) * S_B + pc * 128, ch), yv[i], X3);   // lo copy: blocks 2, 3
-      if (ROLE == 0) { dbs.x += yv[i].x; dbs.y += yv[i].y; dbs.z += yv[i].z; dbs.w += yv[i].w; }
-    }
-  };
-
-  if (ROLE == 1) {
-    // columns 0 and 17 of the skip blocks are never written by `store`; the unused dx = -1 / +1 second halves read
-    // them, and although those accumulators are discarded they must not hold NaN/Inf garbage that an exception-free
-    // tensor core would still multiply: zero both stages' operand regions once
-    for (uint32_t o = tid * 16; o < 2 * STAGE; o += kThreads * 16) *reinterpret_cast<float4*>(smem + o) = make_float4(0.f, 0.f, 0.f, 0.f);
-    __syncthreads();
-  }
-  if (t_begin < t_end) fetch(t_begin);
-  long long it = 0;
-  for (long long tile = t_begin; tile < t_end; ++tile, ++it) {
-    const int s = (int)(it & 1);
-    uint8_t* st = smem + s * STAGE;
-    if (it >= 2) mbar_wait(bars + s, (uint32_t)(((it >> 1) - 1) & 1));   // the MMAs of tile it-2 have read this stage
-    store(st);
-    fence_proxy_async();
-    __syncthreads();
-    if (warp_u == 0) {   // all 32 lanes run the loop (descriptors stay in uniform registers), the elected lane issues
-      tc_fence_after();
-      const uint32_t a_hi = smem_u32(st), a_lo = a_hi + A_PLANE, b0 = a_hi + 2 * A_PLANE;
-#pragma unroll 1
-      for (int r = 0; r < RT; ++r) {
-#pragma unroll
-        for (int hf = 0; hf < 2; ++hf) {
-          const uint64_t bd = mn_desc(b0 + r * 4 * S_B + hf * 8 * 128, S_B);
-#pragma unroll
-          for (int j = 0; j < 3; ++j) {   // dx = j - 1: the (halo) column of output pixel k is hf*8 + k + j
-            const uint32_t aoff = r * ROW_A + (hf * 8 + j) * 128;
-            const uint32_t d = tmem + j * 128;
-            const uint32_t acc = (it == 0 && r == 0 && hf == 0) ? 0u : 1u;
-            if (X3) {
-              umma_tf32(d, mn_desc(a_hi + aoff, S_A), bd, kIdesc128x128, acc, leader);
-              umma_tf32(d + 64, mn_desc(a_lo + aoff, S_A), bd, kIdesc128x64, 1u, leader);
-            } else {
-              umma_tf32(d, mn_desc(a_hi + aoff, S_A), bd, kIdesc128x64, acc, leader);
-            }
-          }
-        }
-      }
-      umma_commit(bars + s, leader);
-      if (tile + 1 == t_end) umma_commit(bars + 2, leader);
-    }
-    if (tile + 1 < t_end) fetch(tile + 1);
-  }
-  // every chunk has at least one tile (the host sizes `per` that way)
-  mbar_wait(bars + 2, 0);
-  tc_fence_after();
-  if (ROLE == 0 && a.part_db) {   // all MMAs have retired: the stages are free for the 16-row reduction of the dY sums
-    float* red = reinterpret_cast<float*>(smem);
-    *reinterpret_cast<float4*>(red + (tid >> 4) * 64 + c16 * 4) = dbs;
-    __syncthreads();
-    if (tid < 64) {
-      float t = 0.f;
-#pragma unroll
-      for (int r = 0; r < 16; ++r) t += red[r * 64 + tid];
-      a.part_db[(long long)chunk * 64 + tid] = t;
-    }
-  }
-  // rows m = 32 q + lane = half_tap * 64 + ci; warps w and w + 4 share lane quarter q = w % 4 and take 32 co each
-  const int q = warp & 3, half = warp >> 2, second = q >> 1, ci = (q & 1) * 32 + lane;
-#pragma unroll 1
-  for (int j = 0; j < 3; ++j) {
-    int tap;
-    if (ROLE == 0) tap = second * 3 + j;                                // (dy = -1 | 0, dx = j - 1)
-    else tap = second ? ((j == 1 && a.ntaps > 9) ? 9 : -1) : 6 + j;     // (dy = +1, dx = j - 1) | the skip tap
-    uint32_t r0[32], r1[32];
-    const uint32_t ta = tmem + (static_cast<uint32_t>(q * 32) << 16) + j * 128 + half * 32;
-    tmem_ld32(ta, r0);                 // warp-collective: every warp reads, only valid taps are written
-    if (X3) tmem_ld32(ta + 64, r1);
-    if (tap >= 0) {
-      float* po = a.part + ((long long)chunk * a.ntaps + tap) * 64 * 64 + ci;
-#pragma unroll
-      for (int i = 0; i < 32; ++i)
-        po[(half * 32 + i) * 64] = (X3 ? __uint_as_float(r1[i]) : 0.f) + __uint_as_float(r0[i]);   // lanes = consecutive ci
-    }
-  }
-}
-
-template <bool X3>
-__global__ void __launch_bounds__(kThreads, 1) tapwgrad_halo_kernel(const HaloWgradArgs a) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + 2 * STAGE);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 4);
-  const int tid = threadIdx.x, warp = tid >> 5;
-  if (tid == 0) {
-    mbar_init(bars + 0, 1);   // stage 0 drained by the tensor core
-    mbar_init(bars + 1, 1);   // stage 1
-    mbar_init(bars + 2, 1);   // all MMAs of the chunk retired
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(tmem_slot)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *tmem_slot;
-  if (blockIdx.y == 0) run_role<X3, 0>(a, smem, bars, tmem);
-  else run_role<X3, 1>(a, smem, bars, tmem);
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem) : "memory");
-}
-
-// ------------------------------------------------------------------------------------------------------------
-// TMA-fed, warp-specialised variant (default).  Same planes, descriptors, roles, accumulators and partial layout as
-// tapwgrad_halo_kernel; what changes is who moves the data and who waits for whom:
-//   warp 8      loader: per tile one cp.async.bulk.tensor per (row, 32-channel block) of the x halo, the skip rows and
-//               the dY tile drops the raw fp32 pixels into the `hi` regions of a stage (4-D maps [channel][x][y][image],
-//               box 32 x pixels x 1 x 1, SWIZZLE_128B_ATOM_32B = the MN-major operand swizzle; image borders arrive as
-//               zeros) -- no global load, no address arithmetic in any thread;
-//   warps 0-7   split warps, shared memory -> shared memory: hi = rn_tf32(x) in place, lo = x - hi to the `lo` region
-//               (the same operand bits as the register-staged kernel), and the dY column sums for the bias gradient;
-//   warp 9      MMA issuer only: full/empty mbarriers hand stages over, so the tensor core works on tile i while the
-//               loader and the split warps prepare tile i+1 (in the block-synchronous kernel warp 0 issued a tile's 48
-//               MMAs and then helped stage the next one: T_tile = T_issue + T_store).
-// ------------------------------------------------------------------------------------------------------------
 struct HaloWgradTma {
   tma::Map x;     // [64][W][H][N]  box 32 x 18 x 1 x 1
   tma::Map dy;    // [64][W][H][N]  box 32 x 16 x 1 x 1
   tma::Map xs;    // parity-(0,0) view of the skip source [64][W][H][N] (strides doubled), box 32 x 16 x 1 x 1
 };
-constexpr int kSplitThreads = 256, kLoadWarp = 8, kIssueWarp = 9, kThreadsTma = 320;
+constexpr int kSplitThreads = 256, kLoadWarp = 8, kIssueWarp = 9, kThreads = 320;
 
 __device__ __forceinline__ float4 lds128(uint32_t saddr) {
   float4 v;
@@ -353,7 +162,7 @@ __device__ __forceinline__ void run_role_tma(const HaloWgradArgs& a, const HaloW
   if (ROLE == 1) {
     // columns 0 and 17 of the skip blocks are never written; the unused second halves of the dx = -1 / +1 pairs read
     // them, so they must not hold NaN / Inf garbage: zero both stages once (before any tensor copy is issued)
-    for (uint32_t o = tid * 16; o < 2 * STAGE; o += kThreadsTma * 16) *reinterpret_cast<float4*>(smem + o) = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (uint32_t o = tid * 16; o < 2 * STAGE; o += kThreads * 16) *reinterpret_cast<float4*>(smem + o) = make_float4(0.f, 0.f, 0.f, 0.f);
     fence_proxy_async();
     __syncthreads();
   }
@@ -481,8 +290,8 @@ __device__ __forceinline__ void run_role_tma(const HaloWgradArgs& a, const HaloW
 }
 
 template <bool X3>
-__global__ void __launch_bounds__(kThreadsTma, 1) tapwgrad_halo_tma_kernel(const HaloWgradArgs a,
-                                                                            const __grid_constant__ HaloWgradTma tm) {
+__global__ void __launch_bounds__(kThreads, 1) tapwgrad_halo_tma_kernel(const HaloWgradArgs a,
+                                                                         const __grid_constant__ HaloWgradTma tm) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + 2 * STAGE);
@@ -501,7 +310,7 @@ __global__ void __launch_bounds__(kThreadsTma, 1) tapwgrad_halo_tma_kernel(const
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = *tmem_slot;
-  if ((a.only_role < 0 ? (int)blockIdx.y : a.only_role) == 0) run_role_tma<X3, 0>(a, tm, smem, bars, tmem);
+  if (blockIdx.y == 0) run_role_tma<X3, 0>(a, tm, smem, bars, tmem);
   else run_role_tma<X3, 1>(a, tm, smem, bars, tmem);
   tc_fence_before();
   __syncthreads();
@@ -554,7 +363,7 @@ __device__ __forceinline__ void run_role_s2(const HaloWgradArgs& a, const HaloWg
   float4 dbs = make_float4(0.f, 0.f, 0.f, 0.f);
 
   if (ROLE == 1) {   // the unused second half of the (0,0) single reads beyond region Z: keep it finite
-    for (uint32_t o = tid * 16; o < NST * STAGE2; o += kThreadsTma * 16) *reinterpret_cast<float4*>(smem + o) = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (uint32_t o = tid * 16; o < NST * STAGE2; o += kThreads * 16) *reinterpret_cast<float4*>(smem + o) = make_float4(0.f, 0.f, 0.f, 0.f);
     fence_proxy_async();
     __syncthreads();
   }
@@ -684,8 +493,8 @@ __device__ __forceinline__ void run_role_s2(const HaloWgradArgs& a, const HaloWg
 }
 
 template <bool X3>
-__global__ void __launch_bounds__(kThreadsTma, 1) tapwgrad_halo_s2_kernel(const HaloWgradArgs a,
-                                                                           const __grid_constant__ HaloWgradS2Tma tm) {
+__global__ void __launch_bounds__(kThreads, 1) tapwgrad_halo_s2_kernel(const HaloWgradArgs a,
+                                                                        const __grid_constant__ HaloWgradS2Tma tm) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + s2::NST * s2::STAGE2);
@@ -736,13 +545,8 @@ int launch_s2(const HaloWgradArgs& h, int chunks, cudaStream_t st) {
       return B200NP_E_LAUNCH;
     configured = true;
   }
-  tapwgrad_halo_s2_kernel<X3><<<dim3(chunks, 2), kThreadsTma, smem, st>>>(h, tm);
+  tapwgrad_halo_s2_kernel<X3><<<dim3(chunks, 2), kThreads, smem, st>>>(h, tm);
   return launch_status();
-}
-
-static bool wgrad_tma_enabled() {
-  static const bool on = [] { const char* e = getenv("B200NP_WGRAD_TMA"); return e ? e[0] != '0' : true; }();
-  return on;
 }
 
 template <bool X3>
@@ -767,20 +571,7 @@ int launch_tma(const HaloWgradArgs& h, int chunks, cudaStream_t st) {
       return B200NP_E_LAUNCH;
     configured = true;
   }
-  tapwgrad_halo_tma_kernel<X3><<<dim3(chunks, h.only_role < 0 ? 2 : 1), kThreadsTma, smem, st>>>(h, tm);
-  return launch_status();
-}
-
-template <bool X3>
-int launch(const HaloWgradArgs& h, int chunks, cudaStream_t st) {
-  const size_t smem = 2 * STAGE + 1024 + 1024;
-  static bool configured = false;
-  if (!configured) {
-    if (cudaFuncSetAttribute(tapwgrad_halo_kernel<X3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-      return B200NP_E_LAUNCH;
-    configured = true;
-  }
-  tapwgrad_halo_kernel<X3><<<dim3(chunks, 2), kThreads, smem, st>>>(h);
+  tapwgrad_halo_tma_kernel<X3><<<dim3(chunks, 2), kThreads, smem, st>>>(h, tm);
   return launch_status();
 }
 
@@ -802,7 +593,7 @@ int tapwgrad_halo_s2_chunks(int N, int OH, int OW) {
   return (int)ceil_div(tiles, per);
 }
 static int launch_tapwgrad_halo_s2(TapWgradArgs& a, int precision, cudaStream_t st) {
-  if (!wgrad_tma_enabled() || a.ntaps != 9 || a.srcH != 2 * a.OH || a.srcW != 2 * a.OW) return B200NP_E_UNSUPPORTED;
+  if (a.ntaps != 9 || a.srcH != 2 * a.OH || a.srcW != 2 * a.OW) return B200NP_E_UNSUPPORTED;
   for (int t = 0; t < 9; ++t)
     if (a.taps[t].src != 0 || a.taps[t].dy != t / 3 - 1 || a.taps[t].dx != t % 3 - 1) return B200NP_E_UNSUPPORTED;
   const int chunks = tapwgrad_halo_s2_chunks(a.N, a.OH, a.OW);
@@ -810,7 +601,7 @@ static int launch_tapwgrad_halo_s2(TapWgradArgs& a, int precision, cudaStream_t 
   HaloWgradArgs h{};
   h.x = a.src; h.dy = a.dy; h.xs = nullptr;
   h.part = a.part; h.part_db = a.part_db;
-  h.N = a.N; h.H = a.OH; h.W = a.OW; h.ntaps = 9; h.only_role = -1;
+  h.N = a.N; h.H = a.OH; h.W = a.OW; h.ntaps = 9;
   h.tiles = (long long)a.N * (a.OH / s2::RT2) * (a.OW / TW);
   h.per = ceil_div(h.tiles, kNumSMs);
   const int rc = precision == B200NP_PREC_TF32 ? launch_s2<false>(h, chunks, st) : launch_s2<true>(h, chunks, st);
@@ -836,14 +627,9 @@ int launch_tapwgrad_halo(TapWgradArgs& a, int precision, cudaStream_t st) {
   h.N = a.N; h.H = a.OH; h.W = a.OW; h.ntaps = a.ntaps;
   h.tiles = (long long)a.N * (a.OH / RT) * (a.OW / TW);
   h.per = ceil_div(h.tiles, kNumSMs);
-  static const int only_role = [] { const char* e = getenv("B200NP_WGRAD_ONLY_ROLE"); return (e && e[0]) ? atoi(e) : -1; }();
-  h.only_role = only_role;
-  a.chunks = chunks;
-  if (wgrad_tma_enabled()) {
-    const int rc = precision == B200NP_PREC_TF32 ? launch_tma<false>(h, chunks, st) : launch_tma<true>(h, chunks, st);
-    if (rc != B200NP_E_UNSUPPORTED) return rc;
-  }
-  return precision == B200NP_PREC_TF32 ? launch<false>(h, chunks, st) : launch<true>(h, chunks, st);
+  const int rc = precision == B200NP_PREC_TF32 ? launch_tma<false>(h, chunks, st) : launch_tma<true>(h, chunks, st);
+  if (rc == B200NP_OK) a.chunks = chunks;
+  return rc;
 }
 
 }  // namespace b200np
