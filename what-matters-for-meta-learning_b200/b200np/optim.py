@@ -27,6 +27,8 @@ class FlatParams:
     def __init__(self, module, dead=lambda name: ".resnet.fc." in name, late=lambda name: name.startswith(FlatParams.LATE),
                  trigger=lambda name: name in FlatParams.TRIGGER):
         named = list(module.named_parameters())
+        index = {n: i for i, (n, _) in enumerate(named)}
+        self.names = [n for n, _ in named]    # in module.parameters() order, the order optimizer checkpoints use
         alive = [(n, p) for n, p in named if not dead(n)]
         live = [(n, p) for n, p in alive if not late(n)] + [(n, p) for n, p in alive if late(n)]
         rest = [(n, p) for n, p in named if dead(n)]
@@ -38,6 +40,7 @@ class FlatParams:
         self.flat = torch.zeros(total, device=dev, dtype=torch.float32)
         self.grad = torch.zeros(self.n_live, device=dev, dtype=torch.float32)
         self.live, self.views, self._keep = [], {}, []
+        self.live_index = []                  # position in module.parameters() of each entry of self.live
         off = 0
         for n, p in live + rest:
             k = p.numel()
@@ -46,6 +49,7 @@ class FlatParams:
             p.data = view
             if off < self.n_live:
                 self.live.append((n, p, off, k))
+                self.live_index.append(index[n])
             off += pad(k)
         self.trigger_ptrs = {p.data_ptr() for n, p, _, _ in self.live if trigger(n)}
 
@@ -166,6 +170,85 @@ class FusedAdam:
         ops.adam_step_dev(f.flat, f.grad, self.m, self.v, f.n_live, self.lr, self.betas[0], self.betas[1], self.eps,
                           self.wd, self.t_dev, 1.0 / world)
 
+    # the rest of a torch.optim.Adam param_group, at the values that describe what the fused kernel computes
+    _GROUP_FLAGS = dict(amsgrad=False, maximize=False, foreach=None, capturable=False, differentiable=False, fused=None,
+                        decoupled_weight_decay=False)
+
+    def state_dict(self):
+        """The optimizer state in exactly the structure `torch.optim.Adam(model.parameters()).state_dict()` has, so
+        either optimizer can resume from the other's checkpoint.  `state` is keyed by position in
+        `module.parameters()`; each live parameter gets `step` (0-dim float32 CPU tensor) and clones of its slices
+        of the moments.  Parameters that never receive a gradient, and every parameter before the first step, get
+        no entry, as in torch.  Reading the step count is one 4-byte device-to-host copy."""
+        f = self.flat
+        t = int(self.t_dev.item())
+        state = {}
+        if t > 0:
+            for i, (_, p, off, k) in sorted(zip(f.live_index, f.live), key=lambda e: e[0]):
+                state[i] = {"step": torch.tensor(float(t), dtype=torch.float32),
+                            "exp_avg": self.m[off:off + k].view_as(p).clone(),
+                            "exp_avg_sq": self.v[off:off + k].view_as(p).clone()}
+        group = dict(lr=self.lr, betas=tuple(self.betas), eps=self.eps, weight_decay=self.wd, **self._GROUP_FLAGS,
+                     params=list(range(len(f.names))))
+        return {"state": state, "param_groups": [group]}
+
+    def load_state_dict(self, state_dict):
+        """Resume from a `state_dict()` of this class or of `torch.optim.Adam` over the same model's parameters.
+
+        The moments are written into the existing `m` / `v` (one `multi_copy` launch per 64 parameters) and the step
+        count into `t_dev`, all in place, so a CUDA graph captured over these buffers stays valid.  A parameter
+        without a state entry gets zero moments.  The hyperparameters are taken from the checkpoint, as torch does.
+        The whole checkpoint is checked before anything is written; `ValueError` if it does not fit this model or
+        needs something the flat kernel does not do (one step counter, plain Adam)."""
+        f = self.flat
+        groups = state_dict["param_groups"]
+        if len(groups) != 1:
+            raise ValueError(f"FusedAdam has one parameter group; the checkpoint has {len(groups)}")
+        group = groups[0]
+        for flag in ("amsgrad", "maximize", "decoupled_weight_decay"):
+            if group.get(flag, False):
+                raise ValueError(f"the checkpoint was written with {flag}=True; FusedAdam implements plain Adam only")
+        ids = list(group["params"])
+        if len(ids) != len(f.names):
+            raise ValueError(f"the checkpoint holds {len(ids)} parameters, the model has {len(f.names)}")
+        live = dict(zip(f.live_index, f.live))
+        found, steps = {}, set()
+        for i, pid in enumerate(ids):
+            s = state_dict["state"].get(pid)
+            if s is None:
+                continue
+            name = f.names[i]
+            if i not in live:
+                raise ValueError(f"the checkpoint has Adam state for {name!r}, which never receives a gradient here")
+            shape = tuple(live[i][1].shape)
+            for key in ("exp_avg", "exp_avg_sq"):
+                if tuple(s[key].shape) != shape:
+                    raise ValueError(f"{name}: the checkpoint's {key} has shape {tuple(s[key].shape)}, "
+                                     f"the parameter {shape}")
+            steps.add(float(s["step"]))
+            found[i] = s
+        if len(steps) > 1:
+            raise ValueError(f"the parameters' Adam step counts differ ({sorted(steps)}); the fused kernel keeps one "
+                             "step counter for all of them")
+        t = steps.pop() if steps else 0.0
+        if t < 0 or t != int(t) or t >= 2 ** 31:
+            raise ValueError(f"Adam step count {t} is not a valid int32 count")
+        dev = f.grad.device
+        seg_m, seg_v = [], []
+        for i, (_, p, off, k) in zip(f.live_index, f.live):
+            s = found.get(i)
+            if s is None:
+                seg_m.append((None, off, k)), seg_v.append((None, off, k))
+            else:
+                seg_m.append((s["exp_avg"].detach().to(dev, torch.float32).contiguous(), off, k))
+                seg_v.append((s["exp_avg_sq"].detach().to(dev, torch.float32).contiguous(), off, k))
+        ops.multi_copy(self.m, seg_m)
+        ops.multi_copy(self.v, seg_v)
+        self.t_dev.fill_(int(t))
+        self.t = int(t)
+        self.lr, self.eps, self.wd = float(group["lr"]), float(group["eps"]), float(group["weight_decay"])
+        self.betas = tuple(float(b) for b in group["betas"])
+
 
 class GraphedStep:
     """One meta-train step (zero_grad, forward, loss, backward, all-reduce, Adam) captured in a CUDA graph.
@@ -182,7 +265,9 @@ class GraphedStep:
 
     Building a graph runs `warmup` real steps and the capture itself on the model; parameters, Adam moments and
     the step counter are snapshotted before and restored afterwards, so constructing the object (or meeting a new
-    shape) does NOT advance training.
+    shape) does NOT advance training.  A graph holds the Adam hyperparameters it was captured with; when `opt.lr`,
+    `betas`, `eps` or `wd` have changed since (by assignment or `load_state_dict`), the graph is recaptured, in the
+    same way, before its next replay.
 
     Input pipeline: ``step(batch, next_batch=...)`` starts the host-to-device copy of the NEXT batch on a
     second stream into staging buffers while this step computes (the reference gets the same overlap from
@@ -212,6 +297,10 @@ class GraphedStep:
     def _key(batch):
         return tuple(tuple(t.shape) for t in batch)
 
+    def _hyper(self):
+        o = self.opt
+        return (o.lr, tuple(o.betas), o.eps, o.wd)
+
     def _entry(self, batch):
         key = self._key(batch)
         ent = self.cache.get(key)
@@ -222,7 +311,14 @@ class GraphedStep:
                "stage": [torch.empty(t.shape, device=dev, dtype=t.dtype) for t in batch]}
         for s, t in zip(ent["static"], batch):
             s.copy_(t)
+        self._capture(ent)
+        self.cache[key] = ent
+        return ent
+
+    def _capture(self, ent):
+        """Warm up and capture the step on `ent`'s static inputs, recording the hyperparameters the graph holds."""
         opt = self.opt
+        old = ent.get("graph")
         snap = (opt.flat.flat.clone(), opt.m.clone(), opt.v.clone(), opt.t_dev.clone(), opt.t)
         cur = torch.cuda.current_stream()
         self.side.wait_stream(cur)
@@ -238,9 +334,9 @@ class GraphedStep:
         opt.flat.flat.copy_(snap[0]), opt.m.copy_(snap[1]), opt.v.copy_(snap[2]), opt.t_dev.copy_(snap[3])
         opt.t = snap[4]
         torch.cuda.synchronize()
-        ent["graph"], ent["loss"] = graph, loss
-        self.cache[key] = ent
-        return ent
+        ent["graph"], ent["loss"], ent["hyper"] = graph, loss, self._hyper()
+        if old is not None and self.graph is old:     # recaptured the example batch's graph
+            self.graph, self.loss = graph, loss
 
     def _eager(self, static):
         cx, cy, tx, ty = static
@@ -276,6 +372,10 @@ class GraphedStep:
             for s, t in zip(ent["static"], batch):
                 if s.data_ptr() != t.data_ptr():
                     s.copy_(t, non_blocking=True)
+        if ent["hyper"] != self._hyper():
+            # the Adam launch in the graph carries the hyperparameters as kernel arguments: a graph captured before
+            # `opt.lr = ...` or `load_state_dict` would silently keep the old values
+            self._capture(ent)
         self._staged = None
         self.ev_free.record(cur)
         ent["graph"].replay()
@@ -283,6 +383,17 @@ class GraphedStep:
         if next_batch is not None:
             self.prefetch(next_batch)
         return ent["loss"]
+
+    def state_dict(self):
+        """What a resumed run needs: `{"model": model.state_dict(), "optimizer": opt.state_dict()}`."""
+        return {"model": self.model.state_dict(), "optimizer": self.opt.state_dict()}
+
+    def load_state_dict(self, state_dict):
+        """Load weights and optimizer state in place (the captured graphs keep their buffers; a graph whose
+        hyperparameters changed is recaptured before its next replay).  The optimizer goes first: it checks the
+        checkpoint against the model's parameters before anything is written."""
+        self.opt.load_state_dict(state_dict["optimizer"])
+        self.model.load_state_dict(state_dict["model"])
 
 
 class GraphedEval:
