@@ -293,6 +293,21 @@ int b200np_adam_step(float* p, const float* g, float* m, float* v, long long n, 
 int b200np_adam_step_dev(float* p, const float* g, float* m, float* v, long long n, float lr, float beta1,
                          float beta2, float eps, float weight_decay, int* step_dev, float grad_scale,
                          void* stream);
+/* out[0] (device) = scale * ||g||_2 over n >= 1 floats (torch.nn.utils.clip_grad_norm_'s total norm).  fp64 partial
+ * sums in a fixed order over a grid that depends on n only: bitwise repeatable.  The partials go to the caller's
+ * workspace of b200np_grad_norm_workspace(n) bytes (8-byte aligned), so calls on different workspaces may run
+ * concurrently.  out[0] is finite exactly when every element of g is (a finite norm beyond FLT_MAX saturates). */
+size_t b200np_grad_norm_workspace(long long n);
+int b200np_grad_norm(const float* g, long long n, float scale, float* out, void* ws, size_t ws_bytes, void* stream);
+/* b200np_adam_step_dev with the learning rate read from device memory (*lr) and, optionally, gradient clipping and
+ * non-finite step skipping decided on the device from `norm`, the b200np_grad_norm of g with scale = grad_scale:
+ *   max_norm (nullable): the scaled gradient is multiplied by min(1, *max_norm / (*norm + 1e-6)), clip_grad_norm_'s
+ *     coefficient (a NaN norm gives a NaN coefficient, as there);
+ *   skipped (nullable): when *norm is not finite, p, m, v and *step_dev are left unchanged and *skipped is incremented.
+ * With both NULL (norm is then ignored) the results are bit-identical to b200np_adam_step_dev with lr = *lr. */
+int b200np_adam_step_ctrl(float* p, const float* g, float* m, float* v, long long n, const float* lr, float beta1,
+                          float beta2, float eps, float weight_decay, int* step_dev, float grad_scale,
+                          const float* max_norm, const float* norm, int* skipped, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * MMAML conv nets (SURVEY.md 8f-3): GatedConvModel (networks/gated_conv_net.py:167-212: 3x3 stride-2 conv ->

@@ -375,6 +375,26 @@ def adam_step_dev(p, g, m, v, n, lr, b1, b2, eps, wd, step_dev, grad_scale=1.0):
                                    grad_scale, _stream()), "adam_step_dev")
 
 
+def grad_norm_workspace(n, like):
+    """The workspace `grad_norm` takes for an n-float segment, on `like`'s device."""
+    return torch.empty(LIB.b200np_grad_norm_workspace(n), device=like.device, dtype=torch.uint8)
+
+
+def grad_norm(g, n, out, ws, scale=1.0):
+    """out[0] = scale * ||g[:n]||_2 (fp64 sums, bitwise repeatable); `ws` from grad_norm_workspace."""
+    _chk(g, "g"), _chk(out, "out")
+    check(LIB.b200np_grad_norm(_ptr(g), n, scale, _ptr(out), _ptr(ws), ws.numel(), _stream()), "grad_norm")
+
+
+def adam_step_ctrl(p, g, m, v, n, lr, b1, b2, eps, wd, step_dev, grad_scale=1.0, max_norm=None, norm=None,
+                   skipped=None):
+    """adam_step_dev with lr a device scalar; clipping to the device scalar `max_norm` and skipping a non-finite step
+    (counted in `skipped`) are decided from `norm` = grad_norm(g, scale=grad_scale).  None switches either off."""
+    check(LIB.b200np_adam_step_ctrl(_ptr(p), _ptr(g), _ptr(m), _ptr(v), n, _ptr(lr), b1, b2, eps, wd, _ptr(step_dev),
+                                    grad_scale, _ptr(max_norm), _ptr(norm), _ptr(skipped), _stream()),
+          "adam_step_ctrl")
+
+
 # ----------------------------------------------------------------------------------------------
 # MMAML conv nets (SURVEY.md 8f-3): im2col / col2im for 3x3 stride-2 convs, batch-stat norm + scale/shift + ReLU
 # ----------------------------------------------------------------------------------------------

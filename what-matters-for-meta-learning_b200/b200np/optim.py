@@ -29,6 +29,7 @@ class FlatParams:
         named = list(module.named_parameters())
         index = {n: i for i, (n, _) in enumerate(named)}
         self.names = [n for n, _ in named]    # in module.parameters() order, the order optimizer checkpoints use
+        self.params = [p for _, p in named]
         alive = [(n, p) for n, p in named if not dead(n)]
         live = [(n, p) for n, p in alive if not late(n)] + [(n, p) for n, p in alive if late(n)]
         rest = [(n, p) for n, p in named if dead(n)]
@@ -92,9 +93,36 @@ class FlatParams:
             p.grad = None
 
 
-class FusedAdam:
+class _Group(dict):
+    """FusedAdam's parameter group.  Assigning "lr" -- by a torch LR scheduler, `opt.lr = x` or `load_state_dict` --
+    also writes the device scalar the Adam kernel reads: one small launch, no synchronisation, and captured graphs
+    see the new value on their next replay."""
+
+    def __init__(self, lr_dev, **kw):
+        super().__init__(**kw)
+        self.lr_dev = lr_dev
+
+    def __setitem__(self, key, value):
+        if key == "lr":
+            self.lr_dev.fill_(value)
+        super().__setitem__(key, value)
+
+
+class FusedAdam(torch.optim.Optimizer):
     """torch.optim.Adam semantics (train.py:52-56: lr from config, betas (0.9, 0.999), eps 1e-8,
     optional L2 weight decay) as one kernel over the flat live-parameter segment.
+
+    A `torch.optim.Optimizer` with one parameter group over `module.parameters()`, so that the schedulers of
+    `torch.optim.lr_scheduler` drive it.  The learning rate lives on the device (see `_Group`); `betas`, `eps` and
+    `weight_decay` are kernel arguments.
+
+    `max_grad_norm`: clip the gradient to this total norm, as `torch.nn.utils.clip_grad_norm_` between `backward()`
+    and `step()` would, but after the data-parallel all-reduce (the norm is that of the averaged gradient, the same on
+    every rank).  The clip coefficient is applied inside the Adam kernel, so `.grad` keeps the UNCLIPPED gradient.
+    `skip_nonfinite`: a step whose gradient holds an inf or NaN leaves the parameters, both moments and the step count
+    unchanged and adds one to `skipped_steps`.  With either set, `grad_norm` is the pre-clip total norm of the last
+    step, as `clip_grad_norm_` returns it; both are device tensors, so reading them needs no per-step
+    synchronisation.  `max_grad_norm` is a device value too: changing it reaches captured graphs without a recapture.
 
     Data parallel (world size > 1): the gradient exchange runs as TWO buckets.  When the encoder CNN's backward starts
     (engine.PRE_TRUNK_BACKWARD_HOOKS) every other gradient is complete: they are gathered and all-reduced on a second
@@ -102,14 +130,24 @@ class FusedAdam:
     bytes) follows at the end, and the Adam kernel waits for both.  Inside a captured step this is a graph branch.
     `B200NP_BUCKETS=0`: one all-reduce after the backward pass."""
 
-    def __init__(self, flat: FlatParams, lr=1e-4, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0):
+    def __init__(self, flat: FlatParams, lr=1e-4, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, max_grad_norm=None,
+                 skip_nonfinite=False):
         import os
         import weakref
-        self.flat, self.lr, self.betas, self.eps, self.wd = flat, lr, betas, eps, weight_decay
+        dev = flat.grad.device
+        defaults = dict(lr=lr, betas=tuple(betas), eps=eps, weight_decay=weight_decay, **self._GROUP_FLAGS)
+        super().__init__([_Group(torch.zeros((), device=dev), params=flat.params)], defaults)
+        self.lr = lr                          # add_param_group's setdefault does not reach the device scalar
+        self.flat = flat
         self.m = torch.zeros_like(flat.grad)
         self.v = torch.zeros_like(flat.grad)
-        self.t = 0
-        self.t_dev = torch.zeros(1, device=flat.grad.device, dtype=torch.int32)  # step count for graph replay
+        self.t = 0                            # host count of step() calls and replays, skipped steps included
+        self.t_dev = torch.zeros(1, device=dev, dtype=torch.int32)  # Adam's step count: the kernels read this one
+        self._max_norm_dev = torch.zeros((), device=dev)
+        self.max_grad_norm, self.skip_nonfinite = max_grad_norm, bool(skip_nonfinite)
+        self.grad_norm = torch.zeros((), device=dev)
+        self.skipped_steps = torch.zeros((), device=dev, dtype=torch.int32)
+        self._norm_ws = ops.grad_norm_workspace(flat.n_live, flat.grad)
         self._early_done, self._early_keep, self._comm = False, [], None
         if os.environ.get("B200NP_BUCKETS", "1") != "0" and flat.n_early and flat.n_early < flat.n_live:
             from . import engine
@@ -122,6 +160,48 @@ class FusedAdam:
                 elif ptr in me.flat.trigger_ptrs:
                     me._early_bucket()
             engine.PRE_TRUNK_BACKWARD_HOOKS.append(hook)
+
+    @property
+    def lr(self):
+        return self.param_groups[0]["lr"]
+
+    @lr.setter
+    def lr(self, value):
+        self.param_groups[0]["lr"] = value
+
+    @property
+    def betas(self):
+        return tuple(self.param_groups[0]["betas"])
+
+    @betas.setter
+    def betas(self, value):
+        self.param_groups[0]["betas"] = tuple(value)
+
+    @property
+    def eps(self):
+        return self.param_groups[0]["eps"]
+
+    @eps.setter
+    def eps(self, value):
+        self.param_groups[0]["eps"] = value
+
+    @property
+    def wd(self):
+        return self.param_groups[0]["weight_decay"]
+
+    @wd.setter
+    def wd(self, value):
+        self.param_groups[0]["weight_decay"] = value
+
+    @property
+    def max_grad_norm(self):
+        return self._max_grad_norm
+
+    @max_grad_norm.setter
+    def max_grad_norm(self, value):
+        if value is not None:
+            self._max_norm_dev.fill_(float(value))
+        self._max_grad_norm = value
 
     def zero_grad(self, set_to_none=False):
         self.flat.zero_grad()
@@ -166,9 +246,15 @@ class FusedAdam:
             if world > 1:
                 dist.all_reduce_grads(f.grad)
         self.t += 1
-        # the step counter is kept on the device so that a captured CUDA graph of the whole step stays valid
-        ops.adam_step_dev(f.flat, f.grad, self.m, self.v, f.n_live, self.lr, self.betas[0], self.betas[1], self.eps,
-                          self.wd, self.t_dev, 1.0 / world)
+        # the step counter, the learning rate and the clip / skip decision are kept on the device so that a captured
+        # CUDA graph of the whole step stays valid
+        clip = self.max_grad_norm is not None
+        if clip or self.skip_nonfinite:
+            ops.grad_norm(f.grad, f.n_live, self.grad_norm, self._norm_ws, 1.0 / world)
+        b1, b2 = self.betas
+        ops.adam_step_ctrl(f.flat, f.grad, self.m, self.v, f.n_live, self.param_groups[0].lr_dev, b1, b2, self.eps,
+                           self.wd, self.t_dev, 1.0 / world, max_norm=self._max_norm_dev if clip else None,
+                           norm=self.grad_norm, skipped=self.skipped_steps if self.skip_nonfinite else None)
 
     # the rest of a torch.optim.Adam param_group, at the values that describe what the fused kernel computes
     _GROUP_FLAGS = dict(amsgrad=False, maximize=False, foreach=None, capturable=False, differentiable=False, fused=None,
@@ -179,7 +265,8 @@ class FusedAdam:
         either optimizer can resume from the other's checkpoint.  `state` is keyed by position in
         `module.parameters()`; each live parameter gets `step` (0-dim float32 CPU tensor) and clones of its slices
         of the moments.  Parameters that never receive a gradient, and every parameter before the first step, get
-        no entry, as in torch.  Reading the step count is one 4-byte device-to-host copy."""
+        no entry, as in torch.  Keys a scheduler added to the group (`initial_lr`) are carried along.  Reading the
+        step count is one 4-byte device-to-host copy."""
         f = self.flat
         t = int(self.t_dev.item())
         state = {}
@@ -188,7 +275,8 @@ class FusedAdam:
                 state[i] = {"step": torch.tensor(float(t), dtype=torch.float32),
                             "exp_avg": self.m[off:off + k].view_as(p).clone(),
                             "exp_avg_sq": self.v[off:off + k].view_as(p).clone()}
-        group = dict(lr=self.lr, betas=tuple(self.betas), eps=self.eps, weight_decay=self.wd, **self._GROUP_FLAGS,
+        group = {k: v for k, v in self.param_groups[0].items() if k != "params"}
+        group.update(lr=float(self.lr), betas=self.betas, eps=self.eps, weight_decay=self.wd, **self._GROUP_FLAGS,
                      params=list(range(len(f.names))))
         return {"state": state, "param_groups": [group]}
 
@@ -197,7 +285,8 @@ class FusedAdam:
 
         The moments are written into the existing `m` / `v` (one `multi_copy` launch per 64 parameters) and the step
         count into `t_dev`, all in place, so a CUDA graph captured over these buffers stays valid.  A parameter
-        without a state entry gets zero moments.  The hyperparameters are taken from the checkpoint, as torch does.
+        without a state entry gets zero moments.  The hyperparameters are taken from the checkpoint, as torch does,
+        and so are the extra group keys a scheduler keeps there (`initial_lr`).
         The whole checkpoint is checked before anything is written; `ValueError` if it does not fit this model or
         needs something the flat kernel does not do (one step counter, plain Adam)."""
         f = self.flat
@@ -246,6 +335,11 @@ class FusedAdam:
         ops.multi_copy(self.v, seg_v)
         self.t_dev.fill_(int(t))
         self.t = int(t)
+        g = self.param_groups[0]
+        own = {"params", "param_names", "lr", "betas", "eps", "weight_decay", *self._GROUP_FLAGS}
+        for k in [k for k in g if k not in own]:
+            del g[k]
+        g.update((k, v) for k, v in group.items() if k not in own)
         self.lr, self.eps, self.wd = float(group["lr"]), float(group["eps"]), float(group["weight_decay"])
         self.betas = tuple(float(b) for b in group["betas"])
 
@@ -263,11 +357,12 @@ class GraphedStep:
     shapes (at most `max_ctx_num` entries) and built on first use; all of them share one memory pool, because they
     never run concurrently.
 
-    Building a graph runs `warmup` real steps and the capture itself on the model; parameters, Adam moments and
-    the step counter are snapshotted before and restored afterwards, so constructing the object (or meeting a new
-    shape) does NOT advance training.  A graph holds the Adam hyperparameters it was captured with; when `opt.lr`,
-    `betas`, `eps` or `wd` have changed since (by assignment or `load_state_dict`), the graph is recaptured, in the
-    same way, before its next replay.
+    Building a graph runs `warmup` real steps and the capture itself on the model; parameters, Adam moments, the
+    step counter and the skip counter are snapshotted before and restored afterwards, so constructing the object (or
+    meeting a new shape) does NOT advance training.  The learning rate and `max_grad_norm` are read from device
+    memory, so a scheduler changes them without a recapture.  A graph holds `betas`, `eps` and `wd` as kernel
+    arguments, and whether clipping and skipping are on; when these have changed since the capture (by assignment,
+    a scheduler or `load_state_dict`), the graph is recaptured, in the same way, before its next replay.
 
     Input pipeline: ``step(batch, next_batch=...)`` starts the host-to-device copy of the NEXT batch on a
     second stream into staging buffers while this step computes (the reference gets the same overlap from
@@ -299,7 +394,7 @@ class GraphedStep:
 
     def _hyper(self):
         o = self.opt
-        return (o.lr, tuple(o.betas), o.eps, o.wd)
+        return (o.betas, o.eps, o.wd, o.max_grad_norm is not None, o.skip_nonfinite)
 
     def _entry(self, batch):
         key = self._key(batch)
@@ -319,7 +414,8 @@ class GraphedStep:
         """Warm up and capture the step on `ent`'s static inputs, recording the hyperparameters the graph holds."""
         opt = self.opt
         old = ent.get("graph")
-        snap = (opt.flat.flat.clone(), opt.m.clone(), opt.v.clone(), opt.t_dev.clone(), opt.t)
+        snap = (opt.flat.flat.clone(), opt.m.clone(), opt.v.clone(), opt.t_dev.clone(), opt.t,
+                opt.skipped_steps.clone(), opt.grad_norm.clone())
         cur = torch.cuda.current_stream()
         self.side.wait_stream(cur)
         with torch.cuda.stream(self.side):
@@ -333,6 +429,7 @@ class GraphedStep:
         # neither the warm-up steps nor the capture may advance training
         opt.flat.flat.copy_(snap[0]), opt.m.copy_(snap[1]), opt.v.copy_(snap[2]), opt.t_dev.copy_(snap[3])
         opt.t = snap[4]
+        opt.skipped_steps.copy_(snap[5]), opt.grad_norm.copy_(snap[6])
         torch.cuda.synchronize()
         ent["graph"], ent["loss"], ent["hyper"] = graph, loss, self._hyper()
         if old is not None and self.graph is old:     # recaptured the example batch's graph
@@ -373,13 +470,14 @@ class GraphedStep:
                 if s.data_ptr() != t.data_ptr():
                     s.copy_(t, non_blocking=True)
         if ent["hyper"] != self._hyper():
-            # the Adam launch in the graph carries the hyperparameters as kernel arguments: a graph captured before
-            # `opt.lr = ...` or `load_state_dict` would silently keep the old values
+            # the Adam launch in the graph carries betas / eps / wd as kernel arguments: a graph captured before they
+            # changed would silently keep the old values
             self._capture(ent)
         self._staged = None
         self.ev_free.record(cur)
         ent["graph"].replay()
         self.opt.t += 1
+        self.opt._opt_called = True    # a replay is an optimizer step: torch's LR schedulers check for one
         if next_batch is not None:
             self.prefetch(next_batch)
         return ent["loss"]

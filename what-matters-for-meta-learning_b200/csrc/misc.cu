@@ -1,4 +1,5 @@
 // Elementwise / reduction kernels: HBM-bound, coalesced, vectorised where alignment allows.
+#include <float.h>
 #include <math.h>
 
 #include "common.cuh"
@@ -685,6 +686,81 @@ extern "C" int b200np_loss_fwd_bwd(const float* mu, const float* y, float* loss,
 }
 
 // ------------------------------------------------------------------------------------------------
+// Total gradient norm over a flat segment: out = scale * ||g||_2.  A grid that depends on n only, per-thread fp64 sums in
+// a fixed order, fixed-shape block trees, and a one-block second stage over the partials in the caller's workspace: the
+// result is bitwise repeatable, and two calls with different workspaces may run concurrently.  fp64 sums of squares of
+// finite fp32 values cannot overflow, so the result is finite exactly when every element is.
+// ------------------------------------------------------------------------------------------------
+constexpr int kNormThreads = 256;
+constexpr long long kNormBlocks = 4 * kNumSMs;
+static long long norm_blocks(long long n) {
+  long long b = ceil_div(ceil_div(n, 4), kNormThreads);
+  return b < kNormBlocks ? b : kNormBlocks;
+}
+__device__ __forceinline__ double block_sum_f64(double v, double* red) {
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  if (lane == 0) red[w] = v;
+  __syncthreads();
+  double t = lane < nw ? red[lane] : 0.0;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
+  return t;
+}
+__global__ void __launch_bounds__(kNormThreads) grad_norm_partial_kernel(const float* __restrict__ g, long long n, int vec,
+                                                                         double* __restrict__ part) {
+  __shared__ double red[32];
+  const long long st = (long long)gridDim.x * blockDim.x;
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  double acc = 0.0;
+  long long tail = i;
+  if (vec) {
+    const long long n4 = n >> 2;
+    for (long long k = i; k < n4; k += st) {
+      const float4 x = __ldg(reinterpret_cast<const float4*>(g) + k);
+      acc = fma((double)x.x, (double)x.x, acc);
+      acc = fma((double)x.y, (double)x.y, acc);
+      acc = fma((double)x.z, (double)x.z, acc);
+      acc = fma((double)x.w, (double)x.w, acc);
+    }
+    tail = (n4 << 2) + i;
+  }
+  for (long long k = tail; k < n; k += st) {
+    const double x = __ldg(g + k);
+    acc = fma(x, x, acc);
+  }
+  acc = block_sum_f64(acc, red);
+  if (threadIdx.x == 0) part[blockIdx.x] = acc;
+}
+__global__ void __launch_bounds__(kNormThreads) grad_norm_finish_kernel(const double* __restrict__ part, int nparts,
+                                                                        float scale, float* __restrict__ out) {
+  __shared__ double red[32];
+  double s = 0.0;
+  for (int b = threadIdx.x; b < nparts; b += blockDim.x) s += part[b];
+  s = block_sum_f64(s, red);
+  if (threadIdx.x == 0) {
+    const double r = sqrt(s) * (double)scale;
+    // a finite norm beyond the fp32 range saturates, so that out[0] is finite exactly when every element is
+    out[0] = isfinite(r) ? (float)fmin(r, (double)FLT_MAX) : (float)r;
+  }
+}
+extern "C" size_t b200np_grad_norm_workspace(long long n) {
+  return n > 0 ? (size_t)norm_blocks(n) * sizeof(double) : 0;
+}
+extern "C" int b200np_grad_norm(const float* g, long long n, float scale, float* out, void* ws, size_t ws_bytes,
+                                void* stream) {
+  if (!g || !out || n <= 0) return B200NP_E_BADARG;
+  if (!ws || ws_bytes < b200np_grad_norm_workspace(n)) return B200NP_E_WORKSPACE;
+  if (reinterpret_cast<uintptr_t>(ws) & 7u) return B200NP_E_BADARG;
+  const long long blocks = norm_blocks(n);
+  double* part = static_cast<double*>(ws);
+  grad_norm_partial_kernel<<<(unsigned)blocks, kNormThreads, 0, as_stream(stream)>>>(g, n, aligned16(g), part);
+  grad_norm_finish_kernel<<<1, kNormThreads, 0, as_stream(stream)>>>(part, (int)blocks, scale, out);
+  return launch_status(2);
+}
+
+// ------------------------------------------------------------------------------------------------
 // Fused Adam on a flat segment: 16 B read + 12 B written per parameter, float4 vectorised.
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void adam_one(float& p, float g, float& m, float& v, float b1, float b2, float eps,
@@ -696,12 +772,36 @@ __device__ __forceinline__ void adam_one(float& p, float g, float& m, float& v, 
   float denom = sqrtf(v) * inv_bc2_sqrt + eps;
   p = p - step_size * (m / denom);
 }
-__global__ void adam_tick_kernel(int* step) { *step += 1; }
+// Device-resident controls of b200np_adam_step_ctrl.  lr == nullptr: none, the kernel takes lr from its argument.
+struct AdamCtrl {
+  const float* lr;
+  const float* max_norm;  // nullable: no clipping
+  const float* norm;      // b200np_grad_norm of the same (grad_scale-scaled) gradient
+  int skip;               // leave everything unchanged when *norm is not finite
+};
+__device__ __forceinline__ bool adam_skips(const float* norm, bool skip) { return skip && !isfinite(__ldg(norm)); }
+// the step counter ticks unless the step is skipped; a skipped step ticks `skipped` instead
+__global__ void adam_tick_kernel(int* step, const float* norm, int* skipped) {
+  if (adam_skips(norm, skipped != nullptr))
+    *skipped += 1;
+  else
+    *step += 1;
+}
 
 __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                             float* __restrict__ v, long long n, float b1, float b2, float eps, float wd,
                             float step_size, float inv_bc2_sqrt, float gs, int vec, const int* __restrict__ step_dev,
-                            float lr) {
+                            float lr, AdamCtrl ctrl) {
+  if (ctrl.lr) {
+    if (adam_skips(ctrl.norm, ctrl.skip)) return;
+    lr = __ldg(ctrl.lr);
+    if (ctrl.max_norm) {
+      // torch.nn.utils.clip_grad_norm_'s coefficient, NaN included; folded into the scale, which it leaves unchanged
+      // when it is 1
+      const float c = __ldg(ctrl.max_norm) / (__ldg(ctrl.norm) + 1e-6f);
+      gs *= c >= 1.f ? 1.f : c;
+    }
+  }
   if (step_dev) {  // CUDA-graph friendly: the step count lives on the device, bias corrections are derived here
     const double t = (double)__ldg(step_dev);
     step_size = (float)((double)lr / (1.0 - pow((double)b1, t)));
@@ -740,7 +840,7 @@ extern "C" int b200np_adam_step(float* p, const float* g, float* m, float* v, lo
   float inv_bc2_sqrt = (float)(1.0 / sqrt(bc2));
   int vec = aligned16(p) && aligned16(g) && aligned16(m) && aligned16(v);
   adam_kernel<<<ew_grid((n + 3) / 4, 256), 256, 0, as_stream(stream)>>>(
-      p, g, m, v, n, beta1, beta2, eps, weight_decay, step_size, inv_bc2_sqrt, grad_scale, vec, nullptr, lr);
+      p, g, m, v, n, beta1, beta2, eps, weight_decay, step_size, inv_bc2_sqrt, grad_scale, vec, nullptr, lr, AdamCtrl{});
   return launch_status();
 }
 
@@ -750,8 +850,22 @@ extern "C" int b200np_adam_step_dev(float* p, const float* g, float* m, float* v
   if (n <= 0) return B200NP_OK;
   if (!p || !g || !m || !v || !step_dev) return B200NP_E_BADARG;
   int vec = aligned16(p) && aligned16(g) && aligned16(m) && aligned16(v);
-  adam_tick_kernel<<<1, 1, 0, as_stream(stream)>>>(step_dev);
+  adam_tick_kernel<<<1, 1, 0, as_stream(stream)>>>(step_dev, nullptr, nullptr);
   adam_kernel<<<ew_grid((n + 3) / 4, 256), 256, 0, as_stream(stream)>>>(p, g, m, v, n, beta1, beta2, eps, weight_decay,
-                                                                        0.f, 0.f, grad_scale, vec, step_dev, lr);
+                                                                        0.f, 0.f, grad_scale, vec, step_dev, lr, AdamCtrl{});
+  return launch_status(2);
+}
+
+extern "C" int b200np_adam_step_ctrl(float* p, const float* g, float* m, float* v, long long n, const float* lr,
+                                     float beta1, float beta2, float eps, float weight_decay, int* step_dev,
+                                     float grad_scale, const float* max_norm, const float* norm, int* skipped,
+                                     void* stream) {
+  if (n <= 0) return B200NP_OK;
+  if (!p || !g || !m || !v || !lr || !step_dev || ((max_norm || skipped) && !norm)) return B200NP_E_BADARG;
+  int vec = aligned16(p) && aligned16(g) && aligned16(m) && aligned16(v);
+  adam_tick_kernel<<<1, 1, 0, as_stream(stream)>>>(step_dev, norm, skipped);
+  adam_kernel<<<ew_grid((n + 3) / 4, 256), 256, 0, as_stream(stream)>>>(
+      p, g, m, v, n, beta1, beta2, eps, weight_decay, 0.f, 0.f, grad_scale, vec, step_dev, 0.f,
+      AdamCtrl{lr, max_norm, norm, skipped != nullptr});
   return launch_status(2);
 }
