@@ -308,6 +308,24 @@ int b200np_grad_norm(const float* g, long long n, float scale, float* out, void*
 int b200np_adam_step_ctrl(float* p, const float* g, float* m, float* v, long long n, const float* lr, float beta1,
                           float beta2, float eps, float weight_decay, int* step_dev, float grad_scale,
                           const float* max_norm, const float* norm, int* skipped, void* stream);
+/* One parameter group of b200np_adam_step_groups: one record per group in device memory. */
+typedef struct {
+  float lr, weight_decay, beta1, beta2, eps;
+  int decoupled; /* 0: L2 decay, g += weight_decay p (torch.optim.Adam);
+                    1: p *= 1 - lr weight_decay before the update (torch.optim.AdamW) */
+} b200np_adam_group;
+/* b200np_adam_step_ctrl over parameter groups, in one launch (plus the step tick).  Every hyperparameter is read from
+ * the device table `groups` (n_groups records, 1..1024), so a write to it reaches a captured graph.  The segment is
+ * cut into n_runs runs: run r is [run_begin[r], run_begin[r + 1]) and belongs to group run_group[r], or to no group
+ * when run_group[r] is negative or >= n_groups (frozen: neither read nor written).  Preconditions the call cannot check
+ * without synchronising: run_begin (n_runs + 1 device int64) ascends strictly from 0 to n in multiples of 4.
+ * n % 4 == 0 and p, g, m, v are 16-B aligned (else B200NP_E_BADARG).  The bias corrections of each group come from
+ * *step_dev and the group's betas.  Clipping and skipping as in b200np_adam_step_ctrl, with `norm` the norm of the
+ * whole segment, frozen runs included.  A group table holding one group over one run gives results bit-identical to
+ * b200np_adam_step_ctrl. */
+int b200np_adam_step_groups(float* p, const float* g, float* m, float* v, long long n, const b200np_adam_group* groups,
+                            int n_groups, const long long* run_begin, const int* run_group, int n_runs, int* step_dev,
+                            float grad_scale, const float* max_norm, const float* norm, int* skipped, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * MMAML conv nets (SURVEY.md 8f-3): GatedConvModel (networks/gated_conv_net.py:167-212: 3x3 stride-2 conv ->

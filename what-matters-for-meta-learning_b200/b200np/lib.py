@@ -73,6 +73,7 @@ SIGNATURES = {
     "b200np_grad_norm_workspace": (_sz, [_ll]),
     "b200np_grad_norm": (_i, [_p, _ll, _f, _p, _p, _sz, _p]),
     "b200np_adam_step_ctrl": (_i, [_p, _p, _p, _p, _ll, _p, _f, _f, _f, _f, _p, _f, _p, _p, _p, _p]),
+    "b200np_adam_step_groups": (_i, [_p, _p, _p, _p, _ll, _p, _i, _p, _p, _i, _p, _f, _p, _p, _p, _p]),
     "b200np_im2col3x3s2": (_i, [_p, _p, _i, _i, _i, _i, _p]),
     "b200np_col2im3x3s2": (_i, [_p, _p, _p, _i, _i, _i, _i, _p]),
     "b200np_im2col_small": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _i, _p]),

@@ -395,6 +395,35 @@ def adam_step_ctrl(p, g, m, v, n, lr, b1, b2, eps, wd, step_dev, grad_scale=1.0,
           "adam_step_ctrl")
 
 
+ADAM_GROUP_FIELDS = ("lr", "weight_decay", "beta1", "beta2", "eps", "decoupled")   # b200np_adam_group, 4 B each
+
+
+def adam_group_table(groups, device):
+    """The device table b200np_adam_step_groups reads: a float32 [len(groups), 6] tensor, one b200np_adam_group per
+    row, from dicts with torch.optim.Adam's keys.  The `decoupled` column holds an int32 (write it through
+    `.view(torch.int32)`)."""
+    rows = torch.tensor([[g["lr"], g["weight_decay"], *g["betas"], g["eps"], 0.0] for g in groups], dtype=F32)
+    rows.view(torch.int32)[:, 5] = torch.tensor([int(bool(g["decoupled_weight_decay"])) for g in groups],
+                                                dtype=torch.int32)
+    return rows.to(device)
+
+
+def adam_step_groups(p, g, m, v, n, groups, run_begin, run_group, step_dev, grad_scale=1.0, max_norm=None, norm=None,
+                     skipped=None):
+    """adam_step_ctrl with every hyperparameter read per parameter group from the device table `groups`
+    (adam_group_table).  Run r of the segment, [run_begin[r], run_begin[r + 1]) (int64, multiples of 4, 0 .. n), is
+    updated with group run_group[r] (int32; -1: frozen, left untouched)."""
+    for t, name in ((p, "p"), (g, "g"), (m, "m"), (v, "v"), (groups, "groups"), (run_group, "run_group")):
+        _chk(t, name)
+    if run_begin.dtype != torch.int64 or not run_begin.is_cuda or run_group.dtype != torch.int32 \
+            or run_begin.numel() != run_group.numel() + 1 or groups.shape[1:] != (len(ADAM_GROUP_FIELDS),):
+        raise lib.B200NPError("adam_step_groups: malformed group or run table")
+    check(LIB.b200np_adam_step_groups(_ptr(p), _ptr(g), _ptr(m), _ptr(v), n, _ptr(groups), groups.shape[0],
+                                      _ptr(run_begin), _ptr(run_group), run_group.numel(), _ptr(step_dev),
+                                      grad_scale, _ptr(max_norm), _ptr(norm), _ptr(skipped), _stream()),
+          "adam_step_groups")
+
+
 # ----------------------------------------------------------------------------------------------
 # MMAML conv nets (SURVEY.md 8f-3): im2col / col2im for 3x3 stride-2 convs, batch-stat norm + scale/shift + ReLU
 # ----------------------------------------------------------------------------------------------

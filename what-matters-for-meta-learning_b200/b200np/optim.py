@@ -94,31 +94,51 @@ class FlatParams:
 
 
 class _Group(dict):
-    """FusedAdam's parameter group.  Assigning "lr" -- by a torch LR scheduler, `opt.lr = x` or `load_state_dict` --
-    also writes the device scalar the Adam kernel reads: one small launch, no synchronisation, and captured graphs
-    see the new value on their next replay."""
+    """One of FusedAdam's parameter groups.  Assigning "lr", "betas", "eps", "weight_decay" or
+    "decoupled_weight_decay" -- by a torch scheduler, `opt.lr = x` or `load_state_dict` -- also writes the group's
+    record of the device table the Adam kernel reads (`row`, see ops.adam_group_table): small fill launches, no
+    synchronisation, and captured graphs see the new value on their next replay.  `row` is None while
+    torch.optim.Optimizer.__init__ builds the group; FusedAdam fills the table afterwards."""
 
-    def __init__(self, lr_dev, **kw):
-        super().__init__(**kw)
-        self.lr_dev = lr_dev
+    _COLUMN = {"lr": 0, "weight_decay": 1, "eps": 4}
+
+    def __init__(self, *args, **kw):
+        super().__init__(*args, **kw)
+        self.row = None
+
+    @property
+    def lr_dev(self):
+        """The device scalar holding this group's learning rate."""
+        return self.row[0]
 
     def __setitem__(self, key, value):
-        if key == "lr":
-            self.lr_dev.fill_(value)
+        if self.row is not None:
+            if key in self._COLUMN:
+                self.row[self._COLUMN[key]].fill_(float(value))
+            elif key == "betas":
+                self.row[2].fill_(float(value[0])), self.row[3].fill_(float(value[1]))
+            elif key == "decoupled_weight_decay":
+                self.row.view(torch.int32)[5].fill_(int(bool(value)))
         super().__setitem__(key, value)
 
 
 class FusedAdam(torch.optim.Optimizer):
-    """torch.optim.Adam semantics (train.py:52-56: lr from config, betas (0.9, 0.999), eps 1e-8,
-    optional L2 weight decay) as one kernel over the flat live-parameter segment.
+    """torch.optim.Adam / AdamW semantics (train.py:52-56: lr from config, betas (0.9, 0.999), eps 1e-8,
+    optional weight decay) as one kernel over the flat live-parameter segment.
 
-    A `torch.optim.Optimizer` with one parameter group over `module.parameters()`, so that the schedulers of
-    `torch.optim.lr_scheduler` drive it.  The learning rate lives on the device (see `_Group`); `betas`, `eps` and
-    `weight_decay` are kernel arguments.
+    A `torch.optim.Optimizer`, so that the schedulers of `torch.optim.lr_scheduler` drive it.  `param_groups=None`:
+    one group over `module.parameters()`.  Otherwise a list of torch-style group dicts (`{"params": [...], "lr": ...,
+    "weight_decay": ..., "decoupled_weight_decay": ...}`; keys a group omits take the constructor's values) over
+    parameters of the flattened module, matched by identity.  A live parameter in no group is frozen, as in torch:
+    never updated, zero moments, no state entry.  The groups are fixed with the flat layout: `add_param_group` after
+    construction raises.  Every hyperparameter of every group lives in a device table (see `_Group`), so changing one
+    needs no recapture of a graph.  `decoupled_weight_decay=True` is AdamW: `p *= 1 - lr * weight_decay` before the
+    update, with the group's current lr.  `opt.lr`, `opt.betas`, `opt.eps` and `opt.wd` are group 0's.
 
     `max_grad_norm`: clip the gradient to this total norm, as `torch.nn.utils.clip_grad_norm_` between `backward()`
     and `step()` would, but after the data-parallel all-reduce (the norm is that of the averaged gradient, the same on
-    every rank).  The clip coefficient is applied inside the Adam kernel, so `.grad` keeps the UNCLIPPED gradient.
+    every rank).  The norm covers every live parameter, frozen ones included, as `clip_grad_norm_(model.parameters())`
+    would.  The clip coefficient is applied inside the Adam kernel, so `.grad` keeps the UNCLIPPED gradient.
     `skip_nonfinite`: a step whose gradient holds an inf or NaN leaves the parameters, both moments and the step count
     unchanged and adds one to `skipped_steps`.  With either set, `grad_norm` is the pre-clip total norm of the last
     step, as `clip_grad_norm_` returns it; both are device tensors, so reading them needs no per-step
@@ -130,14 +150,43 @@ class FusedAdam(torch.optim.Optimizer):
     bytes) follows at the end, and the Adam kernel waits for both.  Inside a captured step this is a graph branch.
     `B200NP_BUCKETS=0`: one all-reduce after the backward pass."""
 
-    def __init__(self, flat: FlatParams, lr=1e-4, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, max_grad_norm=None,
-                 skip_nonfinite=False):
+    def __init__(self, flat: FlatParams, lr=1e-4, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0,
+                 decoupled_weight_decay=False, max_grad_norm=None, skip_nonfinite=False, param_groups=None):
         import os
         import weakref
         dev = flat.grad.device
-        defaults = dict(lr=lr, betas=tuple(betas), eps=eps, weight_decay=weight_decay, **self._GROUP_FLAGS)
-        super().__init__([_Group(torch.zeros((), device=dev), params=flat.params)], defaults)
-        self.lr = lr                          # add_param_group's setdefault does not reach the device scalar
+        defaults = dict(lr=lr, betas=tuple(betas), eps=eps, weight_decay=weight_decay,
+                        decoupled_weight_decay=bool(decoupled_weight_decay), **self._GROUP_FLAGS)
+        groups = [{"params": flat.params}] if param_groups is None else list(param_groups)
+        for g in groups:
+            for flag in ("amsgrad", "maximize"):
+                if g.get(flag, False):
+                    raise ValueError(f"a parameter group sets {flag}=True; FusedAdam implements Adam / AdamW only")
+        super().__init__([_Group(g) for g in groups], defaults)
+        position = {id(p): i for i, p in enumerate(flat.params)}
+        group_of = {}
+        for gi, g in enumerate(self.param_groups):
+            g["betas"] = tuple(g["betas"])
+            for p in g["params"]:
+                if id(p) not in position:
+                    raise ValueError(f"parameter group {gi} holds a tensor of shape {tuple(p.shape)} that is not a "
+                                     "parameter of the flattened module")
+                group_of[position[id(p)]] = gi
+        # the run table: contiguous ranges of flat.flat[:n_live] and their group (-1: frozen); a parameter's padding
+        # belongs to its run, so every run starts at a multiple of 4
+        begin, group = [0], [-1]
+        for i, (_, _, off, _) in zip(flat.live_index, flat.live):
+            gi = group_of.get(i, -1)
+            if group[-1] != gi:
+                begin.append(off), group.append(gi)
+        if len(group) > 1 and begin[1] == 0:      # the first parameter opened a run at 0
+            begin, group = begin[1:], group[1:]
+        begin.append(flat.n_live)
+        self._run_begin = torch.tensor(begin, dtype=torch.int64).to(dev)
+        self._run_group = torch.tensor(group, dtype=torch.int32).to(dev)
+        self._table = ops.adam_group_table(self.param_groups, dev)
+        for g, row in zip(self.param_groups, self._table):
+            g.row = row
         self.flat = flat
         self.m = torch.zeros_like(flat.grad)
         self.v = torch.zeros_like(flat.grad)
@@ -160,6 +209,12 @@ class FusedAdam(torch.optim.Optimizer):
                 elif ptr in me.flat.trigger_ptrs:
                     me._early_bucket()
             engine.PRE_TRUNK_BACKWARD_HOOKS.append(hook)
+
+    def add_param_group(self, param_group):
+        if hasattr(self, "_table"):
+            raise RuntimeError("FusedAdam's parameter groups are fixed at construction (the kernel's run table is laid "
+                               "out with the flat parameters); pass every group to the constructor")
+        super().add_param_group(param_group)
 
     @property
     def lr(self):
@@ -246,63 +301,88 @@ class FusedAdam(torch.optim.Optimizer):
             if world > 1:
                 dist.all_reduce_grads(f.grad)
         self.t += 1
-        # the step counter, the learning rate and the clip / skip decision are kept on the device so that a captured
-        # CUDA graph of the whole step stays valid
+        # the step counter, every hyperparameter and the clip / skip decision are kept on the device so that a
+        # captured CUDA graph of the whole step stays valid
         clip = self.max_grad_norm is not None
         if clip or self.skip_nonfinite:
             ops.grad_norm(f.grad, f.n_live, self.grad_norm, self._norm_ws, 1.0 / world)
-        b1, b2 = self.betas
-        ops.adam_step_ctrl(f.flat, f.grad, self.m, self.v, f.n_live, self.param_groups[0].lr_dev, b1, b2, self.eps,
-                           self.wd, self.t_dev, 1.0 / world, max_norm=self._max_norm_dev if clip else None,
-                           norm=self.grad_norm, skipped=self.skipped_steps if self.skip_nonfinite else None)
+        ops.adam_step_groups(f.flat, f.grad, self.m, self.v, f.n_live, self._table, self._run_begin, self._run_group,
+                             self.t_dev, 1.0 / world, max_norm=self._max_norm_dev if clip else None,
+                             norm=self.grad_norm, skipped=self.skipped_steps if self.skip_nonfinite else None)
 
     # the rest of a torch.optim.Adam param_group, at the values that describe what the fused kernel computes
-    _GROUP_FLAGS = dict(amsgrad=False, maximize=False, foreach=None, capturable=False, differentiable=False, fused=None,
-                        decoupled_weight_decay=False)
+    _GROUP_FLAGS = dict(amsgrad=False, maximize=False, foreach=None, capturable=False, differentiable=False, fused=None)
+    _HYPER = ("lr", "betas", "eps", "weight_decay", "decoupled_weight_decay")
+
+    def _ids(self):
+        """torch's checkpoint numbering: consecutive over the groups' `params` lists, in group order.  Yields
+        (group index, id, position in module.parameters())."""
+        position = {id(p): i for i, p in enumerate(self.flat.params)}
+        k = 0
+        for gi, g in enumerate(self.param_groups):
+            for p in g["params"]:
+                yield gi, k, position[id(p)]
+                k += 1
 
     def state_dict(self):
-        """The optimizer state in exactly the structure `torch.optim.Adam(model.parameters()).state_dict()` has, so
-        either optimizer can resume from the other's checkpoint.  `state` is keyed by position in
-        `module.parameters()`; each live parameter gets `step` (0-dim float32 CPU tensor) and clones of its slices
-        of the moments.  Parameters that never receive a gradient, and every parameter before the first step, get
-        no entry, as in torch.  Keys a scheduler added to the group (`initial_lr`) are carried along.  Reading the
-        step count is one 4-byte device-to-host copy."""
+        """The optimizer state in exactly the structure `torch.optim.Adam(groups).state_dict()` (or `AdamW`) has, so
+        either optimizer can resume from the other's checkpoint.  `state` is keyed by torch's ids (consecutive over
+        the groups' `params`, in group order; for the default single group, the position in `module.parameters()`).
+        Each live parameter of a group gets `step` (0-dim float32 CPU tensor) and clones of its slices of the
+        moments.  Parameters that never receive a gradient, frozen ones, and every parameter before the first step
+        get no entry, as in torch.  Each group carries its own hyperparameters and the keys a scheduler added to it
+        (`initial_lr`).  Reading the step count is one 4-byte device-to-host copy."""
         f = self.flat
         t = int(self.t_dev.item())
+        live = dict(zip(f.live_index, f.live))
         state = {}
         if t > 0:
-            for i, (_, p, off, k) in sorted(zip(f.live_index, f.live), key=lambda e: e[0]):
-                state[i] = {"step": torch.tensor(float(t), dtype=torch.float32),
-                            "exp_avg": self.m[off:off + k].view_as(p).clone(),
-                            "exp_avg_sq": self.v[off:off + k].view_as(p).clone()}
-        group = {k: v for k, v in self.param_groups[0].items() if k != "params"}
-        group.update(lr=float(self.lr), betas=self.betas, eps=self.eps, weight_decay=self.wd, **self._GROUP_FLAGS,
-                     params=list(range(len(f.names))))
-        return {"state": state, "param_groups": [group]}
+            for _, k, i in self._ids():
+                if i in live:
+                    _, p, off, n = live[i]
+                    state[k] = {"step": torch.tensor(float(t), dtype=torch.float32),
+                                "exp_avg": self.m[off:off + n].view_as(p).clone(),
+                                "exp_avg_sq": self.v[off:off + n].view_as(p).clone()}
+        groups, k = [], 0
+        for g in self.param_groups:
+            group = {key: v for key, v in g.items() if key != "params"}
+            group.update(lr=float(g["lr"]), betas=tuple(g["betas"]), eps=g["eps"], weight_decay=g["weight_decay"],
+                         decoupled_weight_decay=bool(g["decoupled_weight_decay"]), **self._GROUP_FLAGS,
+                         params=list(range(k, k + len(g["params"]))))
+            k += len(g["params"])
+            groups.append(group)
+        return {"state": state, "param_groups": groups}
 
     def load_state_dict(self, state_dict):
-        """Resume from a `state_dict()` of this class or of `torch.optim.Adam` over the same model's parameters.
+        """Resume from a `state_dict()` of this class or of `torch.optim.Adam` / `AdamW` over the same parameter
+        groups (same count, same sizes, same order).
 
         The moments are written into the existing `m` / `v` (one `multi_copy` launch per 64 parameters) and the step
         count into `t_dev`, all in place, so a CUDA graph captured over these buffers stays valid.  A parameter
-        without a state entry gets zero moments.  The hyperparameters are taken from the checkpoint, as torch does,
-        and so are the extra group keys a scheduler keeps there (`initial_lr`).
-        The whole checkpoint is checked before anything is written; `ValueError` if it does not fit this model or
-        needs something the flat kernel does not do (one step counter, plain Adam)."""
+        without a state entry gets zero moments.  Each group's hyperparameters are taken from the checkpoint, as torch
+        does, and so are the extra group keys a scheduler keeps there (`initial_lr`).
+        The whole checkpoint is checked before anything is written; `ValueError` if it does not fit these groups or
+        needs something the flat kernel does not do (one step counter, no amsgrad / maximize)."""
         f = self.flat
         groups = state_dict["param_groups"]
-        if len(groups) != 1:
-            raise ValueError(f"FusedAdam has one parameter group; the checkpoint has {len(groups)}")
-        group = groups[0]
-        for flag in ("amsgrad", "maximize", "decoupled_weight_decay"):
-            if group.get(flag, False):
-                raise ValueError(f"the checkpoint was written with {flag}=True; FusedAdam implements plain Adam only")
-        ids = list(group["params"])
-        if len(ids) != len(f.names):
-            raise ValueError(f"the checkpoint holds {len(ids)} parameters, the model has {len(f.names)}")
+        if len(groups) != len(self.param_groups):
+            raise ValueError(f"FusedAdam has {len(self.param_groups)} parameter group(s); the checkpoint has "
+                             f"{len(groups)}")
+        for gi, (group, mine) in enumerate(zip(groups, self.param_groups)):
+            for flag in ("amsgrad", "maximize"):
+                if group.get(flag, False):
+                    raise ValueError(f"the checkpoint was written with {flag}=True; FusedAdam implements Adam / AdamW "
+                                     "only")
+            if len(group["params"]) != len(mine["params"]):
+                raise ValueError(f"parameter group {gi} holds {len(mine['params'])} parameters, the checkpoint's "
+                                 f"{len(group['params'])}")
+        saved = [pid for group in groups for pid in group["params"]]
+        extra = set(state_dict["state"]) - set(saved)
+        if extra:
+            raise ValueError(f"the checkpoint has state for ids {sorted(extra)}, which are in none of its groups")
         live = dict(zip(f.live_index, f.live))
         found, steps = {}, set()
-        for i, pid in enumerate(ids):
+        for (_, k, i), pid in zip(self._ids(), saved):
             s = state_dict["state"].get(pid)
             if s is None:
                 continue
@@ -335,13 +415,15 @@ class FusedAdam(torch.optim.Optimizer):
         ops.multi_copy(self.v, seg_v)
         self.t_dev.fill_(int(t))
         self.t = int(t)
-        g = self.param_groups[0]
-        own = {"params", "param_names", "lr", "betas", "eps", "weight_decay", *self._GROUP_FLAGS}
-        for k in [k for k in g if k not in own]:
-            del g[k]
-        g.update((k, v) for k, v in group.items() if k not in own)
-        self.lr, self.eps, self.wd = float(group["lr"]), float(group["eps"]), float(group["weight_decay"])
-        self.betas = tuple(float(b) for b in group["betas"])
+        own = {"params", "param_names", *self._HYPER, *self._GROUP_FLAGS}
+        for g, group in zip(self.param_groups, groups):
+            for k in [k for k in g if k not in own]:
+                del g[k]
+            g.update((k, v) for k, v in group.items() if k not in own)
+            g["lr"], g["eps"], g["weight_decay"] = float(group["lr"]), float(group["eps"]), float(group["weight_decay"])
+            g["betas"] = tuple(float(b) for b in group["betas"])
+            # a checkpoint older than the key leaves the group's own setting, as torch's Adam / AdamW keep their own
+            g["decoupled_weight_decay"] = bool(group.get("decoupled_weight_decay", g["decoupled_weight_decay"]))
 
 
 class GraphedStep:
@@ -359,10 +441,10 @@ class GraphedStep:
 
     Building a graph runs `warmup` real steps and the capture itself on the model; parameters, Adam moments, the
     step counter and the skip counter are snapshotted before and restored afterwards, so constructing the object (or
-    meeting a new shape) does NOT advance training.  The learning rate and `max_grad_norm` are read from device
-    memory, so a scheduler changes them without a recapture.  A graph holds `betas`, `eps` and `wd` as kernel
-    arguments, and whether clipping and skipping are on; when these have changed since the capture (by assignment,
-    a scheduler or `load_state_dict`), the graph is recaptured, in the same way, before its next replay.
+    meeting a new shape) does NOT advance training.  Every group's hyperparameters and `max_grad_norm` are read from
+    device memory, so a scheduler, an assignment or `load_state_dict` changes them without a recapture.  A graph
+    holds only whether clipping and skipping are on; when that has changed since the capture, the graph is
+    recaptured, in the same way, before its next replay.
 
     Input pipeline: ``step(batch, next_batch=...)`` starts the host-to-device copy of the NEXT batch on a
     second stream into staging buffers while this step computes (the reference gets the same overlap from
@@ -394,7 +476,7 @@ class GraphedStep:
 
     def _hyper(self):
         o = self.opt
-        return (o.betas, o.eps, o.wd, o.max_grad_norm is not None, o.skip_nonfinite)
+        return (o.max_grad_norm is not None, o.skip_nonfinite)
 
     def _entry(self, batch):
         key = self._key(batch)
@@ -470,8 +552,7 @@ class GraphedStep:
                 if s.data_ptr() != t.data_ptr():
                     s.copy_(t, non_blocking=True)
         if ent["hyper"] != self._hyper():
-            # the Adam launch in the graph carries betas / eps / wd as kernel arguments: a graph captured before they
-            # changed would silently keep the old values
+            # the graph holds whether the norm pass runs and what the Adam launch does with it
             self._capture(ent)
         self._staged = None
         self.ev_free.record(cur)
@@ -487,8 +568,8 @@ class GraphedStep:
         return {"model": self.model.state_dict(), "optimizer": self.opt.state_dict()}
 
     def load_state_dict(self, state_dict):
-        """Load weights and optimizer state in place (the captured graphs keep their buffers; a graph whose
-        hyperparameters changed is recaptured before its next replay).  The optimizer goes first: it checks the
+        """Load weights and optimizer state in place: the captured graphs keep their buffers and read the loaded
+        hyperparameters from device memory, so nothing is recaptured.  The optimizer goes first: it checks the
         checkpoint against the model's parameters before anything is written."""
         self.opt.load_state_dict(state_dict["optimizer"])
         self.model.load_state_dict(state_dict["model"])

@@ -762,23 +762,36 @@ extern "C" int b200np_grad_norm(const float* g, long long n, float scale, float*
 
 // ------------------------------------------------------------------------------------------------
 // Fused Adam on a flat segment: 16 B read + 12 B written per parameter, float4 vectorised.
+// One kernel serves every entry point.  Its hyperparameters come from a group table (b200np_adam_step_groups) or from
+// one group passed by value (the single-group entry points); each block derives the per-group bias corrections once
+// into shared memory.  A block updates one contiguous range of the segment, so the run table (which run of the
+// segment belongs to which group) is searched once per thread and then walked forward.
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void adam_one(float& p, float g, float& m, float& v, float b1, float b2, float eps,
-                                         float wd, float step_size, float inv_bc2_sqrt, float gs) {
-  g *= gs;
-  if (wd != 0.f) g = fmaf(wd, p, g);
-  m = m + (g - m) * (1.f - b1);
-  v = v * b2 + (1.f - b2) * g * g;
-  float denom = sqrtf(v) * inv_bc2_sqrt + eps;
-  p = p - step_size * (m / denom);
-}
-// Device-resident controls of b200np_adam_step_ctrl.  lr == nullptr: none, the kernel takes lr from its argument.
-struct AdamCtrl {
-  const float* lr;
-  const float* max_norm;  // nullable: no clipping
-  const float* norm;      // b200np_grad_norm of the same (grad_scale-scaled) gradient
-  int skip;               // leave everything unchanged when *norm is not finite
+struct AdamHyper {
+  float step_size, inv_bc2_sqrt, b1, b2, eps;
+  float wd;     // coupled (L2) decay, folded into the gradient; 0 with decoupled decay
+  float decay;  // decoupled (AdamW) decay: p *= decay before the update; 1 otherwise
 };
+__device__ __forceinline__ void adam_one(float& p, float g, float& m, float& v, const AdamHyper& h, float gs) {
+  g *= gs;
+  if (h.decay != 1.f) p *= h.decay;
+  if (h.wd != 0.f) g = fmaf(h.wd, p, g);
+  m = m + (g - m) * (1.f - h.b1);
+  v = v * h.b2 + (1.f - h.b2) * g * g;
+  float denom = sqrtf(v) * h.inv_bc2_sqrt + h.eps;
+  p = p - h.step_size * (m / denom);
+}
+__device__ __forceinline__ AdamHyper adam_hyper(const b200np_adam_group& G, const int* step_dev, float step_size,
+                                                float inv_bc2_sqrt) {
+  AdamHyper h{step_size, inv_bc2_sqrt, G.beta1, G.beta2, G.eps, G.decoupled ? 0.f : G.weight_decay, 1.f};
+  if (step_dev) {  // CUDA-graph friendly: the step count lives on the device, bias corrections are derived here
+    const double t = (double)__ldg(step_dev);
+    h.step_size = (float)((double)G.lr / (1.0 - pow((double)G.beta1, t)));
+    h.inv_bc2_sqrt = (float)(1.0 / sqrt(1.0 - pow((double)G.beta2, t)));
+  }
+  if (G.decoupled) h.decay = (float)(1.0 - (double)G.lr * (double)G.weight_decay);
+  return h;
+}
 __device__ __forceinline__ bool adam_skips(const float* norm, bool skip) { return skip && !isfinite(__ldg(norm)); }
 // the step counter ticks unless the step is skipped; a skipped step ticks `skipped` instead
 __global__ void adam_tick_kernel(int* step, const float* norm, int* skipped) {
@@ -788,47 +801,109 @@ __global__ void adam_tick_kernel(int* step, const float* norm, int* skipped) {
     *step += 1;
 }
 
-__global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
-                            float* __restrict__ v, long long n, float b1, float b2, float eps, float wd,
-                            float step_size, float inv_bc2_sqrt, float gs, int vec, const int* __restrict__ step_dev,
-                            float lr, AdamCtrl ctrl) {
-  if (ctrl.lr) {
-    if (adam_skips(ctrl.norm, ctrl.skip)) return;
-    lr = __ldg(ctrl.lr);
-    if (ctrl.max_norm) {
-      // torch.nn.utils.clip_grad_norm_'s coefficient, NaN included; folded into the scale, which it leaves unchanged
-      // when it is 1
-      const float c = __ldg(ctrl.max_norm) / (__ldg(ctrl.norm) + 1e-6f);
-      gs *= c >= 1.f ? 1.f : c;
-    }
-  }
-  if (step_dev) {  // CUDA-graph friendly: the step count lives on the device, bias corrections are derived here
-    const double t = (double)__ldg(step_dev);
-    step_size = (float)((double)lr / (1.0 - pow((double)b1, t)));
-    inv_bc2_sqrt = (float)(1.0 / sqrt(1.0 - pow((double)b2, t)));
-  }
-  long long st = (long long)gridDim.x * blockDim.x;
-  long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (vec) {
-    long long n4 = n >> 2;
-    for (long long k = i; k < n4; k += st) {
-      float4 P = reinterpret_cast<float4*>(p)[k], G = reinterpret_cast<const float4*>(g)[k];
-      float4 M = reinterpret_cast<float4*>(m)[k], V = reinterpret_cast<float4*>(v)[k];
-      adam_one(P.x, G.x, M.x, V.x, b1, b2, eps, wd, step_size, inv_bc2_sqrt, gs);
-      adam_one(P.y, G.y, M.y, V.y, b1, b2, eps, wd, step_size, inv_bc2_sqrt, gs);
-      adam_one(P.z, G.z, M.z, V.z, b1, b2, eps, wd, step_size, inv_bc2_sqrt, gs);
-      adam_one(P.w, G.w, M.w, V.w, b1, b2, eps, wd, step_size, inv_bc2_sqrt, gs);
-      reinterpret_cast<float4*>(p)[k] = P;
-      reinterpret_cast<float4*>(m)[k] = M;
-      reinterpret_cast<float4*>(v)[k] = V;
-    }
-    for (long long k = (n4 << 2) + i; k < n; k += st)
-      adam_one(p[k], g[k], m[k], v[k], b1, b2, eps, wd, step_size, inv_bc2_sqrt, gs);
-  } else {
-    for (long long k = i; k < n; k += st)
-      adam_one(p[k], g[k], m[k], v[k], b1, b2, eps, wd, step_size, inv_bc2_sqrt, gs);
-  }
+constexpr int kAdamThreads = 256;
+constexpr int kAdamMaxGroups = 1024;  // shared memory per block: kAdamMaxGroups * sizeof(AdamHyper)
+struct AdamArgs {
+  float* p;
+  const float* g;
+  float* m;
+  float* v;
+  long long n;
+  int vec;                          // every pointer 16-B aligned: float4 units, else single floats
+  float gs;                         // gradient scale (1/world)
+  const int* step_dev;              // nullable: the host bias corrections below are used
+  float step_size, inv_bc2_sqrt;
+  const b200np_adam_group* groups;  // nullable: one group, `one`, over [0, n)
+  int n_groups, n_runs;
+  const long long* run_begin;       // n_runs + 1 float offsets, multiples of 4, from 0 to n
+  const int* run_group;             // group of each run, -1: frozen
+  b200np_adam_group one;
+  const float* lr_dev;              // one group: nullable, replaces one.lr
+  const float* max_norm;            // nullable: no clipping
+  const float* norm;                // b200np_grad_norm of the same (grad_scale-scaled) gradient
+  int skip;                         // leave everything unchanged when *norm is not finite
+};
+
+// the group of run r; a group index outside the table counts as frozen, so a bad table never reads past `hyp`
+__device__ __forceinline__ int adam_run_group(const AdamArgs& a, int r, int ng) {
+  const int grp = __ldg(a.run_group + r);
+  return grp < ng ? grp : -1;
 }
+
+__global__ void __launch_bounds__(kAdamThreads) adam_kernel(const AdamArgs a) {
+  extern __shared__ AdamHyper hyp[];
+  if (adam_skips(a.norm, a.skip)) return;
+  float gs = a.gs;
+  if (a.max_norm) {
+    // torch.nn.utils.clip_grad_norm_'s coefficient, NaN included; folded into the scale, which it leaves unchanged
+    // when it is 1
+    const float c = __ldg(a.max_norm) / (__ldg(a.norm) + 1e-6f);
+    gs *= c >= 1.f ? 1.f : c;
+  }
+  const int ng = a.groups ? a.n_groups : 1;
+  for (int i = threadIdx.x; i < ng; i += blockDim.x) {
+    b200np_adam_group G = a.groups ? a.groups[i] : a.one;
+    if (!a.groups && a.lr_dev) G.lr = __ldg(a.lr_dev);
+    hyp[i] = adam_hyper(G, a.step_dev, a.step_size, a.inv_bc2_sqrt);
+  }
+  __syncthreads();
+
+  const long long nu = a.vec ? a.n >> 2 : a.n;
+  const long long bx = blockDim.x, per = ((nu + gridDim.x - 1) / gridDim.x + bx - 1) / bx * bx;
+  const long long lo = (long long)blockIdx.x * per, hi = lo + per < nu ? lo + per : nu;
+  long long k = lo + threadIdx.x;
+  // the run holding unit k: [run_begin[r], run_begin[r + 1]) in floats, `end` in units
+  int r = 0, grp = 0;
+  long long end = nu;
+  if (a.run_begin && k < hi) {
+    int l = 0, u = a.n_runs - 1;
+    while (l < u) {
+      const int mid = (l + u + 1) >> 1;
+      if (__ldg(a.run_begin + mid) <= 4 * k) l = mid; else u = mid - 1;
+    }
+    r = l;
+    end = __ldg(a.run_begin + r + 1) >> 2;
+    grp = adam_run_group(a, r, ng);
+  }
+  AdamHyper h = hyp[grp < 0 ? 0 : grp];
+  for (; k < hi; k += blockDim.x) {
+    if (k >= end) {
+      do end = __ldg(a.run_begin + (++r) + 1) >> 2; while (k >= end);
+      grp = adam_run_group(a, r, ng);
+      if (grp >= 0) h = hyp[grp];
+    }
+    if (grp < 0) continue;  // frozen: neither read nor written
+    if (a.vec) {
+      float4 P = reinterpret_cast<float4*>(a.p)[k], G = reinterpret_cast<const float4*>(a.g)[k];
+      float4 M = reinterpret_cast<float4*>(a.m)[k], V = reinterpret_cast<float4*>(a.v)[k];
+      adam_one(P.x, G.x, M.x, V.x, h, gs);
+      adam_one(P.y, G.y, M.y, V.y, h, gs);
+      adam_one(P.z, G.z, M.z, V.z, h, gs);
+      adam_one(P.w, G.w, M.w, V.w, h, gs);
+      reinterpret_cast<float4*>(a.p)[k] = P;
+      reinterpret_cast<float4*>(a.m)[k] = M;
+      reinterpret_cast<float4*>(a.v)[k] = V;
+    } else {
+      adam_one(a.p[k], a.g[k], a.m[k], a.v[k], h, gs);
+    }
+  }
+  // the scalar tail of a float4 segment (one group only: a run table needs n % 4 == 0)
+  if (a.vec && blockIdx.x == gridDim.x - 1)
+    for (long long t = (nu << 2) + threadIdx.x; t < a.n; t += blockDim.x)
+      adam_one(a.p[t], a.g[t], a.m[t], a.v[t], hyp[0], gs);
+}
+
+// tick (when `step_dev`) + update; `a` carries everything but the launch shape
+static int adam_launch(AdamArgs a, int* step_dev, int* skipped, void* stream) {
+  a.vec = aligned16(a.p) && aligned16(a.g) && aligned16(a.m) && aligned16(a.v);
+  a.step_dev = step_dev;
+  a.skip = skipped != nullptr;
+  const size_t smem = (size_t)(a.groups ? a.n_groups : 1) * sizeof(AdamHyper);
+  if (step_dev) adam_tick_kernel<<<1, 1, 0, as_stream(stream)>>>(step_dev, a.norm, skipped);
+  adam_kernel<<<ew_grid((a.n + 3) / 4, kAdamThreads), kAdamThreads, smem, as_stream(stream)>>>(a);
+  return launch_status(step_dev ? 2 : 1);
+}
+
 extern "C" int b200np_adam_step(float* p, const float* g, float* m, float* v, long long n, float lr,
                                 float beta1, float beta2, float eps, float weight_decay, int step,
                                 float grad_scale, void* stream) {
@@ -836,12 +911,12 @@ extern "C" int b200np_adam_step(float* p, const float* g, float* m, float* v, lo
   if (!p || !g || !m || !v || step < 1) return B200NP_E_BADARG;
   double bc1 = 1.0 - pow((double)beta1, (double)step);
   double bc2 = 1.0 - pow((double)beta2, (double)step);
-  float step_size = (float)((double)lr / bc1);
-  float inv_bc2_sqrt = (float)(1.0 / sqrt(bc2));
-  int vec = aligned16(p) && aligned16(g) && aligned16(m) && aligned16(v);
-  adam_kernel<<<ew_grid((n + 3) / 4, 256), 256, 0, as_stream(stream)>>>(
-      p, g, m, v, n, beta1, beta2, eps, weight_decay, step_size, inv_bc2_sqrt, grad_scale, vec, nullptr, lr, AdamCtrl{});
-  return launch_status();
+  AdamArgs a{};
+  a.p = p, a.g = g, a.m = m, a.v = v, a.n = n, a.gs = grad_scale;
+  a.step_size = (float)((double)lr / bc1);
+  a.inv_bc2_sqrt = (float)(1.0 / sqrt(bc2));
+  a.one = b200np_adam_group{lr, weight_decay, beta1, beta2, eps, 0};
+  return adam_launch(a, nullptr, nullptr, stream);
 }
 
 extern "C" int b200np_adam_step_dev(float* p, const float* g, float* m, float* v, long long n, float lr,
@@ -849,11 +924,10 @@ extern "C" int b200np_adam_step_dev(float* p, const float* g, float* m, float* v
                                     float grad_scale, void* stream) {
   if (n <= 0) return B200NP_OK;
   if (!p || !g || !m || !v || !step_dev) return B200NP_E_BADARG;
-  int vec = aligned16(p) && aligned16(g) && aligned16(m) && aligned16(v);
-  adam_tick_kernel<<<1, 1, 0, as_stream(stream)>>>(step_dev, nullptr, nullptr);
-  adam_kernel<<<ew_grid((n + 3) / 4, 256), 256, 0, as_stream(stream)>>>(p, g, m, v, n, beta1, beta2, eps, weight_decay,
-                                                                        0.f, 0.f, grad_scale, vec, step_dev, lr, AdamCtrl{});
-  return launch_status(2);
+  AdamArgs a{};
+  a.p = p, a.g = g, a.m = m, a.v = v, a.n = n, a.gs = grad_scale;
+  a.one = b200np_adam_group{lr, weight_decay, beta1, beta2, eps, 0};
+  return adam_launch(a, step_dev, nullptr, stream);
 }
 
 extern "C" int b200np_adam_step_ctrl(float* p, const float* g, float* m, float* v, long long n, const float* lr,
@@ -862,10 +936,25 @@ extern "C" int b200np_adam_step_ctrl(float* p, const float* g, float* m, float* 
                                      void* stream) {
   if (n <= 0) return B200NP_OK;
   if (!p || !g || !m || !v || !lr || !step_dev || ((max_norm || skipped) && !norm)) return B200NP_E_BADARG;
-  int vec = aligned16(p) && aligned16(g) && aligned16(m) && aligned16(v);
-  adam_tick_kernel<<<1, 1, 0, as_stream(stream)>>>(step_dev, norm, skipped);
-  adam_kernel<<<ew_grid((n + 3) / 4, 256), 256, 0, as_stream(stream)>>>(
-      p, g, m, v, n, beta1, beta2, eps, weight_decay, 0.f, 0.f, grad_scale, vec, step_dev, 0.f,
-      AdamCtrl{lr, max_norm, norm, skipped != nullptr});
-  return launch_status(2);
+  AdamArgs a{};
+  a.p = p, a.g = g, a.m = m, a.v = v, a.n = n, a.gs = grad_scale;
+  a.one = b200np_adam_group{0.f, weight_decay, beta1, beta2, eps, 0};
+  a.lr_dev = lr, a.max_norm = max_norm, a.norm = norm;
+  return adam_launch(a, step_dev, skipped, stream);
+}
+
+extern "C" int b200np_adam_step_groups(float* p, const float* g, float* m, float* v, long long n,
+                                       const b200np_adam_group* groups, int n_groups, const long long* run_begin,
+                                       const int* run_group, int n_runs, int* step_dev, float grad_scale,
+                                       const float* max_norm, const float* norm, int* skipped, void* stream) {
+  if (n <= 0) return B200NP_OK;
+  if (!p || !g || !m || !v || !groups || !run_begin || !run_group || !step_dev || ((max_norm || skipped) && !norm))
+    return B200NP_E_BADARG;
+  if (n_groups < 1 || n_groups > kAdamMaxGroups || n_runs < 1 || n % 4) return B200NP_E_BADARG;
+  if (!aligned16(p) || !aligned16(g) || !aligned16(m) || !aligned16(v)) return B200NP_E_BADARG;
+  AdamArgs a{};
+  a.p = p, a.g = g, a.m = m, a.v = v, a.n = n, a.gs = grad_scale;
+  a.groups = groups, a.n_groups = n_groups, a.run_begin = run_begin, a.run_group = run_group, a.n_runs = n_runs;
+  a.max_norm = max_norm, a.norm = norm;
+  return adam_launch(a, step_dev, skipped, stream);
 }
