@@ -200,6 +200,12 @@ int b200np_axpy(float* y, const float* x, long long n, float a, void* stream); /
  * (replaces autograd's per-parameter accumulate kernels).  src / dst_off / numel are HOST arrays. */
 int b200np_multi_copy(const float* const* src, const long long* dst_off, const long long* numel, int nseg,
                       float* dst, void* stream);
+/* dst[dst_off[i] + j] += src[i][j] for nseg segments (a NULL src[i] leaves its range unchanged), with the batching of
+ * b200np_multi_copy: one more micro-batch's gradients added into the flat gradient buffer when gradients are
+ * accumulated over several backward passes.  One fp32 add per element, so the result is deterministic; 16-byte
+ * vectors where src[i] and its destination are both 16-byte aligned.  src / dst_off / numel are HOST arrays. */
+int b200np_multi_accumulate(const float* const* src, const long long* dst_off, const long long* numel, int nseg,
+                            float* dst, void* stream);
 
 /* Device-side task assembly: out [M,C,H,W] fp32 = (255 - bank[rows[m]]) / 255 from a uint8 channel-last image bank
  * [n,H,W,C] resident in HBM (dataset/shapenet_distractor.py:233-234,256-259 + utils/utils.py:26-30: `255 - x`,

@@ -48,6 +48,7 @@ SIGNATURES = {
     "b200np_maxpool2x2_bwd": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _p]),
     "b200np_gather_images_u8": (_i, [_p, _p, _p, _ll, _i, _i, _i, _p]),
     "b200np_multi_copy": (_i, [_p, _p, _p, _i, _p, _p]),
+    "b200np_multi_accumulate": (_i, [_p, _p, _p, _i, _p, _p]),
     "b200np_gemm_workspace": (_sz, [C.POINTER(GemmDesc)]),
     "b200np_gemm": (_i, [C.POINTER(GemmDesc), _p]),
     "b200np_act_bwd": (_i, [_p, _p, _p, _ll, _i, _p]),

@@ -275,15 +275,26 @@ def gather_images_u8(bank, rows, out=None):
     return out
 
 
-def multi_copy(dst, segments):
-    """dst[off:off+n] = src (zeros for src None) for every (src, off, n) in segments -- one launch per 64."""
+def _segments(segments):
+    """(src, off, n) triples -> the host arrays and count of b200np_multi_copy / b200np_multi_accumulate."""
     k = len(segments)
-    if k == 0:
-        return dst
     srcs = (C.c_void_p * k)(*[None if s is None else s.data_ptr() for s, _, _ in segments])
     offs = (C.c_longlong * k)(*[o for _, o, _ in segments])
     nums = (C.c_longlong * k)(*[n for _, _, n in segments])
-    check(LIB.b200np_multi_copy(srcs, offs, nums, k, _ptr(dst), _stream()), "multi_copy")
+    return srcs, offs, nums, k
+
+
+def multi_copy(dst, segments):
+    """dst[off:off+n] = src (zeros for src None) for every (src, off, n) in segments -- one launch per 64."""
+    if segments:
+        check(LIB.b200np_multi_copy(*_segments(segments), _ptr(dst), _stream()), "multi_copy")
+    return dst
+
+
+def multi_accumulate(dst, segments):
+    """dst[off:off+n] += src (src None: left unchanged) for every (src, off, n) in segments -- one launch per 64."""
+    if segments:
+        check(LIB.b200np_multi_accumulate(*_segments(segments), _ptr(dst), _stream()), "multi_accumulate")
     return dst
 
 

@@ -8,6 +8,8 @@ ONE NCCL all-reduce.  Parameters that never receive a gradient (the dead ``resne
 SURVEY.md 8a/a14) are placed after the live ones and skipped, exactly like torch.optim.Adam skips
 ``p.grad is None``.
 """
+import contextlib
+
 import torch
 
 from . import dist, ops
@@ -59,9 +61,11 @@ class FlatParams:
         for _, p, off, k in self.live:
             p.grad = self.grad[off:off + k].view_as(p)
 
-    def gather_grads(self, lo=0, hi=None, keep=None, skip_missing=False):
+    def gather_grads(self, lo=0, hi=None, keep=None, skip_missing=False, accumulate=False):
         """After autograd: bring every .grad with offset in [lo, hi) into the flat buffer -- ONE launch per 64 parameters
         (`b200np_multi_copy`); parameters without a gradient get zeros (`skip_missing`: are left for a later call).
+        `accumulate`: ADD the gradients to what the flat buffer holds (`b200np_multi_accumulate`; the earlier
+        micro-batches of a gradient-accumulation window), and skip parameters without a gradient instead of zeroing.
         Afterwards .grad is the flat view.  `keep`: a list that receives the source tensors (a caller that enqueues the
         copy on another stream keeps them referenced until that stream has joined)."""
         hi = self.n_live if hi is None else hi
@@ -75,14 +79,15 @@ class FlatParams:
             if g is None:
                 if skip_missing:
                     continue
-                segs.append((None, off, k))
+                if not accumulate:
+                    segs.append((None, off, k))
             elif g.data_ptr() != view.data_ptr():
                 if not g.is_contiguous():
                     g = g.contiguous()
                 keep.append(g)            # keep the source alive until the copy has been enqueued
                 segs.append((g, off, k))
             p.grad = view
-        ops.multi_copy(self.grad, segs)
+        (ops.multi_accumulate if accumulate else ops.multi_copy)(self.grad, segs)
         if keep is self._keep:
             self._keep.clear()
 
@@ -148,13 +153,32 @@ class FusedAdam(torch.optim.Optimizer):
     (engine.PRE_TRUNK_BACKWARD_HOOKS) every other gradient is complete: they are gathered and all-reduced on a second
     stream while the encoder CNN's data / weight gradients are still being computed; the CNNs' own bucket (~20 % of the
     bytes) follows at the end, and the Adam kernel waits for both.  Inside a captured step this is a graph branch.
-    `B200NP_BUCKETS=0`: one all-reduce after the backward pass."""
+    `B200NP_BUCKETS=0`: one all-reduce after the backward pass.
+
+    Gradient accumulation (`accumulate_steps=k`, fixed at construction): one `step()` per window of k backward passes,
+    on the SUM of their gradients times 1/(k * world size).  Callers divide the loss by neither k nor the world size.
+    Eagerly, run the window's first k-1 backward passes inside `with opt.no_sync():` and the last one outside, then
+    `step()`; `GraphedStep` does this per call.  Inside `no_sync()` no gradient exchange starts and the gradients sum
+    in `p.grad` under autograd's ordinary rules, so a window costs one exchange whatever k is, and the last backward's
+    early bucket still overlaps the encoder CNN's backward.  On world size > 1 a second backward pass outside
+    `no_sync()` before `step()` raises `RuntimeError` (its gradients would miss the exchange already started).  The
+    norm for clipping and skipping is that of the window's mean gradient, so a NaN in any micro-batch skips the whole
+    step; `t`, `t_dev`, schedulers and `skipped_steps` advance once per window.  `state_dict()` / `load_state_dict()`
+    raise between a window's backward passes: an open window is not part of the saved state.
+    The ANP family's scalar exchanges (the FAVOR+ key stabiliser's MAX in forward, its gradient's SUM in backward) stay
+    per micro-batch: each micro-batch is its own meta-batch for the stabiliser, so k accumulated ANP micro-batches
+    give the sum of their own gradients, not those of one k-times larger meta-batch (SURVEY.md section 0 #5 puts
+    such a difference at 8e-5 relative on the outputs at initialisation).  CNP-family models have independent tasks
+    and a mean loss: k equal-shaped micro-batches of T tasks reproduce one batch of k*T tasks up to fp32 rounding."""
 
     def __init__(self, flat: FlatParams, lr=1e-4, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0,
-                 decoupled_weight_decay=False, max_grad_norm=None, skip_nonfinite=False, param_groups=None):
+                 decoupled_weight_decay=False, max_grad_norm=None, skip_nonfinite=False, param_groups=None,
+                 accumulate_steps=1):
         import os
         import weakref
         dev = flat.grad.device
+        if int(accumulate_steps) != accumulate_steps or accumulate_steps < 1:
+            raise ValueError(f"accumulate_steps={accumulate_steps!r}: needs a whole number of backward passes >= 1")
         defaults = dict(lr=lr, betas=tuple(betas), eps=eps, weight_decay=weight_decay,
                         decoupled_weight_decay=bool(decoupled_weight_decay), **self._GROUP_FLAGS)
         groups = [{"params": flat.params}] if param_groups is None else list(param_groups)
@@ -198,6 +222,10 @@ class FusedAdam(torch.optim.Optimizer):
         self.skipped_steps = torch.zeros((), device=dev, dtype=torch.int32)
         self._norm_ws = ops.grad_norm_workspace(flat.n_live, flat.grad)
         self._early_done, self._early_keep, self._comm = False, [], None
+        self._accumulate_steps = int(accumulate_steps)
+        self._no_sync = False
+        self._micro = 0              # backward passes of the open accumulation window (no_sync blocks / GraphedStep)
+        self._gather_adds = False    # the window's earlier gradients are summed in flat.grad (GraphedStep): gathers add
         if os.environ.get("B200NP_BUCKETS", "1") != "0" and flat.n_early and flat.n_early < flat.n_live:
             from . import engine
             ref = weakref.ref(self)
@@ -206,7 +234,7 @@ class FusedAdam(torch.optim.Optimizer):
                 me = ref()
                 if me is None:
                     engine.PRE_TRUNK_BACKWARD_HOOKS.remove(hook)
-                elif ptr in me.flat.trigger_ptrs:
+                elif ptr in me.flat.trigger_ptrs and not me._no_sync:
                     me._early_bucket()
             engine.PRE_TRUNK_BACKWARD_HOOKS.append(hook)
 
@@ -215,6 +243,22 @@ class FusedAdam(torch.optim.Optimizer):
             raise RuntimeError("FusedAdam's parameter groups are fixed at construction (the kernel's run table is laid "
                                "out with the flat parameters); pass every group to the constructor")
         super().add_param_group(param_group)
+
+    @property
+    def accumulate_steps(self):
+        """Backward passes per optimizer step (fixed at construction)."""
+        return self._accumulate_steps
+
+    @contextlib.contextmanager
+    def no_sync(self):
+        """As DistributedDataParallel.no_sync(): backward passes inside start no gradient exchange, and their gradients
+        sum in `p.grad`.  Run every backward pass of an accumulation window but the last one inside it."""
+        prev, self._no_sync = self._no_sync, True
+        self._micro += 1
+        try:
+            yield
+        finally:
+            self._no_sync = prev
 
     @property
     def lr(self):
@@ -261,18 +305,28 @@ class FusedAdam(torch.optim.Optimizer):
     def zero_grad(self, set_to_none=False):
         self.flat.zero_grad()
         self._early_done = False
+        self._micro, self._gather_adds = 0, False
+
+    def _window_closed(self, what):
+        if self._micro:
+            raise RuntimeError(f"{what}() between the backward passes of a gradient-accumulation window: the window's "
+                               "gradients are not part of the saved state; call it after the window's step()")
 
     def _early_bucket(self):
         """The gradients laid out before the encoder CNN's: gather + all-reduce on the communication stream."""
-        if self._early_done or dist.world_size() == 1:
+        if dist.world_size() == 1:
             return
+        if self._early_done:
+            raise RuntimeError("a second backward pass before step() outside no_sync(): its gradients would miss the "
+                               "exchange the first one started; run all but the last backward pass of a gradient-"
+                               "accumulation window inside `with opt.no_sync():`")
         f = self.flat
         main = torch.cuda.current_stream()
         if self._comm is None:
             self._comm = torch.cuda.Stream(priority=-1)
         self._comm.wait_stream(main)
         with torch.cuda.stream(self._comm):
-            f.gather_grads(0, f.n_early, keep=self._early_keep, skip_missing=True)
+            f.gather_grads(0, f.n_early, keep=self._early_keep, skip_missing=True, accumulate=self._gather_adds)
             dist.all_reduce_sum(f.grad[:f.n_early])
         self._early_done = True
 
@@ -284,6 +338,7 @@ class FusedAdam(torch.optim.Optimizer):
     def _step(self):
         f = self.flat
         world = dist.world_size()
+        acc = self._gather_adds
         if world > 1 and self._early_done:
             # whatever the early bucket did not find (a parameter whose gradient arrived later: none on the shipped
             # models) is exchanged on its own, so the result never depends on the bucket boundary being right
@@ -291,23 +346,25 @@ class FusedAdam(torch.optim.Optimizer):
                           if off < f.n_early and p.grad is not None and p.grad.data_ptr() != f.grad[off:off + k].data_ptr()]
             torch.cuda.current_stream().wait_stream(self._comm)   # before anything else writes into the early segment
             self._early_keep.clear()
-            f.gather_grads()
+            f.gather_grads(accumulate=acc)
             dist.all_reduce_sum(f.grad[f.n_early:f.n_live])
             for _, off, k in late_early:
                 dist.all_reduce_sum(f.grad[off:off + k])
             self._early_done = False
         else:
-            f.gather_grads()
+            f.gather_grads(accumulate=acc)
             if world > 1:
                 dist.all_reduce_grads(f.grad)
         self.t += 1
+        self._micro, self._gather_adds = 0, False
+        scale = 1.0 / (world * self.accumulate_steps)     # the window's mean gradient over every rank
         # the step counter, every hyperparameter and the clip / skip decision are kept on the device so that a
         # captured CUDA graph of the whole step stays valid
         clip = self.max_grad_norm is not None
         if clip or self.skip_nonfinite:
-            ops.grad_norm(f.grad, f.n_live, self.grad_norm, self._norm_ws, 1.0 / world)
+            ops.grad_norm(f.grad, f.n_live, self.grad_norm, self._norm_ws, scale)
         ops.adam_step_groups(f.flat, f.grad, self.m, self.v, f.n_live, self._table, self._run_begin, self._run_group,
-                             self.t_dev, 1.0 / world, max_norm=self._max_norm_dev if clip else None,
+                             self.t_dev, scale, max_norm=self._max_norm_dev if clip else None,
                              norm=self.grad_norm, skipped=self.skipped_steps if self.skip_nonfinite else None)
 
     # the rest of a torch.optim.Adam param_group, at the values that describe what the fused kernel computes
@@ -331,7 +388,9 @@ class FusedAdam(torch.optim.Optimizer):
         Each live parameter of a group gets `step` (0-dim float32 CPU tensor) and clones of its slices of the
         moments.  Parameters that never receive a gradient, frozen ones, and every parameter before the first step
         get no entry, as in torch.  Each group carries its own hyperparameters and the keys a scheduler added to it
-        (`initial_lr`).  Reading the step count is one 4-byte device-to-host copy."""
+        (`initial_lr`).  Reading the step count is one 4-byte device-to-host copy.  Raises between the backward passes
+        of a gradient-accumulation window."""
+        self._window_closed("state_dict")
         f = self.flat
         t = int(self.t_dev.item())
         live = dict(zip(f.live_index, f.live))
@@ -362,7 +421,9 @@ class FusedAdam(torch.optim.Optimizer):
         without a state entry gets zero moments.  Each group's hyperparameters are taken from the checkpoint, as torch
         does, and so are the extra group keys a scheduler keeps there (`initial_lr`).
         The whole checkpoint is checked before anything is written; `ValueError` if it does not fit these groups or
-        needs something the flat kernel does not do (one step counter, no amsgrad / maximize)."""
+        needs something the flat kernel does not do (one step counter, no amsgrad / maximize).  `RuntimeError` between
+        the backward passes of a gradient-accumulation window."""
+        self._window_closed("load_state_dict")
         f = self.flat
         groups = state_dict["param_groups"]
         if len(groups) != len(self.param_groups):
@@ -440,11 +501,20 @@ class GraphedStep:
     never run concurrently.
 
     Building a graph runs `warmup` real steps and the capture itself on the model; parameters, Adam moments, the
-    step counter and the skip counter are snapshotted before and restored afterwards, so constructing the object (or
-    meeting a new shape) does NOT advance training.  Every group's hyperparameters and `max_grad_norm` are read from
-    device memory, so a scheduler, an assignment or `load_state_dict` changes them without a recapture.  A graph
-    holds only whether clipping and skipping are on; when that has changed since the capture, the graph is
-    recaptured, in the same way, before its next replay.
+    step counter, the skip counter, the flat gradient and the position in an accumulation window are snapshotted
+    before and restored afterwards, so constructing the object (or meeting a new shape, mid-window too) does NOT
+    advance training.  Every group's hyperparameters and `max_grad_norm` are read from device memory, so a scheduler,
+    an assignment or `load_state_dict` changes them without a recapture.  A graph holds only whether clipping and
+    skipping are on; when that has changed since the capture, the graph is recaptured, in the same way, before its
+    next replay.
+
+    Gradient accumulation (`opt.accumulate_steps` = k > 1, see FusedAdam): each call is one micro-batch and returns
+    its loss, and the k-th call of a window is the optimizer step.  Per batch shape up to three graphs ("roles") are
+    captured on first use: "first" zeroes the gradients, runs forward, loss and backward and copies the gradients
+    into `flat.grad`; "middle" does the same but adds them; "last" runs forward, loss and backward, adds the gradients
+    and runs the two-bucket exchange, the norm and Adam.  Shapes may differ within a window.  Only "last" graphs hold
+    the clipping / skipping switch, so only they are recaptured when it changes.  With k = 1 the one role is "last",
+    the step described above.
 
     Input pipeline: ``step(batch, next_batch=...)`` starts the host-to-device copy of the NEXT batch on a
     second stream into staging buffers while this step computes (the reference gets the same overlap from
@@ -458,7 +528,7 @@ class GraphedStep:
         self.model, self.lossf, self.opt, self.warmup = model, lossf, opt, warmup
         self.copy_stream = torch.cuda.Stream()
         self.ev_ready, self.ev_free = torch.cuda.Event(), torch.cuda.Event()
-        self._staged = None          # (graph entry, the prefetched batch's tensors)
+        self._staged = None          # (shape entry, the prefetched batch's tensors)
         self.cache = {}
         self.pool = torch.cuda.graph_pool_handle()
         from . import engine
@@ -467,7 +537,7 @@ class GraphedStep:
         self.side = torch.cuda.Stream(priority=engine.MAIN_PRIORITY if engine.USE_PRIORITIES else 0)
         self.graph = self.loss = None
         if example_batch is not None:
-            ent = self._entry(example_batch)
+            ent = self._graph(self._entry(example_batch))
             self.graph, self.loss = ent["graph"], ent["loss"]
 
     @staticmethod
@@ -478,52 +548,78 @@ class GraphedStep:
         o = self.opt
         return (o.max_grad_norm is not None, o.skip_nonfinite)
 
+    def _role(self):
+        """The role of the next call in the accumulation window."""
+        o = self.opt
+        return "last" if o._micro >= o.accumulate_steps - 1 else "middle" if o._micro else "first"
+
     def _entry(self, batch):
+        """The static and staging inputs of `batch`'s shape, with the graph of the next call's role captured."""
         key = self._key(batch)
         ent = self.cache.get(key)
-        if ent is not None:
-            return ent
-        dev = self.opt.flat.flat.device
-        ent = {"static": [torch.empty(t.shape, device=dev, dtype=t.dtype) for t in batch],
-               "stage": [torch.empty(t.shape, device=dev, dtype=t.dtype) for t in batch]}
-        for s, t in zip(ent["static"], batch):
-            s.copy_(t)
-        self._capture(ent)
-        self.cache[key] = ent
+        if ent is None:
+            dev = self.opt.flat.flat.device
+            ent = {"static": [torch.empty(t.shape, device=dev, dtype=t.dtype) for t in batch],
+                   "stage": [torch.empty(t.shape, device=dev, dtype=t.dtype) for t in batch], "roles": {}}
+            for s, t in zip(ent["static"], batch):
+                s.copy_(t)
+            self.cache[key] = ent
+        self._graph(ent)
         return ent
 
+    def _graph(self, ent):
+        """The graph of the next call's role on the shape entry `ent`, captured on first use."""
+        role = self._role()
+        g = ent["roles"].get(role)
+        if g is None:
+            g = ent["roles"][role] = {"static": ent["static"], "role": role}
+            self._capture(g)
+        return g
+
     def _capture(self, ent):
-        """Warm up and capture the step on `ent`'s static inputs, recording the hyperparameters the graph holds."""
-        opt = self.opt
+        """Warm up and capture `ent`'s role on its static inputs, recording the hyperparameters a "last" graph holds."""
+        opt, f = self.opt, self.opt.flat
         old = ent.get("graph")
-        snap = (opt.flat.flat.clone(), opt.m.clone(), opt.v.clone(), opt.t_dev.clone(), opt.t,
-                opt.skipped_steps.clone(), opt.grad_norm.clone())
+        snap = (f.flat.clone(), f.grad.clone(), opt.m.clone(), opt.v.clone(), opt.t_dev.clone(),
+                opt.skipped_steps.clone(), opt.grad_norm.clone(), opt.t, opt._micro, opt._gather_adds)
         cur = torch.cuda.current_stream()
         self.side.wait_stream(cur)
         with torch.cuda.stream(self.side):
             for _ in range(self.warmup):
-                self._eager(ent["static"])
+                self._eager(ent["static"], ent["role"])
         cur.wait_stream(self.side)
         torch.cuda.synchronize()
         graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(graph, stream=self.side, pool=self.pool):
-            loss = self._eager(ent["static"])
-        # neither the warm-up steps nor the capture may advance training
-        opt.flat.flat.copy_(snap[0]), opt.m.copy_(snap[1]), opt.v.copy_(snap[2]), opt.t_dev.copy_(snap[3])
-        opt.t = snap[4]
-        opt.skipped_steps.copy_(snap[5]), opt.grad_norm.copy_(snap[6])
+            loss = self._eager(ent["static"], ent["role"])
+        # neither the warm-up steps nor the capture may advance training or change the open window's gradients
+        for t, saved in zip((f.flat, f.grad, opt.m, opt.v, opt.t_dev, opt.skipped_steps, opt.grad_norm), snap):
+            t.copy_(saved)
+        opt.t, opt._micro, opt._gather_adds = snap[7:]
         torch.cuda.synchronize()
-        ent["graph"], ent["loss"], ent["hyper"] = graph, loss, self._hyper()
+        ent["graph"], ent["loss"] = graph, loss
+        ent["hyper"] = self._hyper() if ent["role"] == "last" else None
         if old is not None and self.graph is old:     # recaptured the example batch's graph
             self.graph, self.loss = graph, loss
 
-    def _eager(self, static):
+    def _eager(self, static, role="last"):
         cx, cy, tx, ty = static
-        self.opt.zero_grad()
+        opt = self.opt
+        if role == "last" and opt.accumulate_steps == 1:
+            opt.zero_grad()
+        else:
+            # autograd hands over this micro-batch's gradients alone; the window's earlier ones are in flat.grad
+            opt.flat.zero_grad()
+            opt._gather_adds = role != "first"
         mu, _, _ = self.model(cx, cy, tx)
         loss = self.lossf.calc_loss(mu, None, ty)
-        loss.backward()
-        self.opt.step()
+        if role == "last":
+            loss.backward()
+            opt.step()
+        else:
+            with opt.no_sync():
+                loss.backward()
+            opt.flat.gather_grads(accumulate=opt._gather_adds)
         return loss.detach()
 
     def prefetch(self, batch):
@@ -551,17 +647,24 @@ class GraphedStep:
             for s, t in zip(ent["static"], batch):
                 if s.data_ptr() != t.data_ptr():
                     s.copy_(t, non_blocking=True)
-        if ent["hyper"] != self._hyper():
+        g = self._graph(ent)
+        if g["hyper"] is not None and g["hyper"] != self._hyper():
             # the graph holds whether the norm pass runs and what the Adam launch does with it
-            self._capture(ent)
+            self._capture(g)
         self._staged = None
         self.ev_free.record(cur)
-        ent["graph"].replay()
-        self.opt.t += 1
-        self.opt._opt_called = True    # a replay is an optimizer step: torch's LR schedulers check for one
+        g["graph"].replay()
+        opt = self.opt
+        if g["role"] == "last":
+            opt.t += 1
+            opt._micro, opt._gather_adds = 0, False
+            opt._opt_called = True     # a replay of the step is an optimizer step: torch's LR schedulers check for one
+        else:
+            opt._micro += 1
+            opt._gather_adds = True
         if next_batch is not None:
             self.prefetch(next_batch)
-        return ent["loss"]
+        return g["loss"]
 
     def state_dict(self):
         """What a resumed run needs: `{"model": model.state_dict(), "optimizer": opt.state_dict()}`."""

@@ -50,24 +50,52 @@ extern "C" int b200np_axpy(float* y, const float* x, long long n, float a, void*
   return launch_status();
 }
 
-// dst[off_i .. off_i + n_i) = src_i (or 0 where src_i is NULL), up to 64 segments per launch, passed by value
+// Segment i of a launch is dst[off_i .. off_i + n_i) and src_i, up to 64 segments per launch, passed by value.
+// kAdd false (copy): dst = src_i, or 0 where src_i is NULL.  kAdd true (accumulate): dst += src_i, and a NULL src_i
+// leaves its range alone; float4 where both sides are 16-byte aligned (always so for FlatParams views), then a scalar
+// tail.  Plain fp32 adds, one per element: deterministic.
 constexpr int kSegsPerLaunch = 64;
 struct CopySegs {
   const float* src[kSegsPerLaunch];
   long long off[kSegsPerLaunch];
   long long n[kSegsPerLaunch];
 };
-__global__ void multi_copy_kernel(const CopySegs g, float* __restrict__ dst) {
-  const float* __restrict__ s = g.src[blockIdx.y];
-  float* __restrict__ d = dst + g.off[blockIdx.y];
-  const long long n = g.n[blockIdx.y];
+template <bool kAdd>
+__device__ __forceinline__ void multi_segment(const float* __restrict__ s, float* __restrict__ d, const long long n) {
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long st = (long long)gridDim.x * blockDim.x;
-  if (s) for (; i < n; i += st) d[i] = s[i];
-  else for (; i < n; i += st) d[i] = 0.f;
+  // __ldg: once this body is inlined, restrict alone no longer gives the read-only loads the copy kernel always had
+  if (!kAdd) {
+    if (s) for (; i < n; i += st) d[i] = __ldg(s + i);
+    else for (; i < n; i += st) d[i] = 0.f;
+    return;
+  }
+  if (!s) return;
+  if (((reinterpret_cast<uintptr_t>(s) | reinterpret_cast<uintptr_t>(d)) & 15) == 0) {
+    const long long n4 = n >> 2;
+    const float4* __restrict__ s4 = reinterpret_cast<const float4*>(s);
+    float4* __restrict__ d4 = reinterpret_cast<float4*>(d);
+    for (long long q = i; q < n4; q += st) {
+      const float4 a = __ldg(s4 + q);
+      float4 b = d4[q];
+      b.x += a.x, b.y += a.y, b.z += a.z, b.w += a.w;
+      d4[q] = b;
+    }
+    i += n4 << 2;
+  }
+  for (; i < n; i += st) d[i] += __ldg(s + i);
 }
-extern "C" int b200np_multi_copy(const float* const* src, const long long* dst_off, const long long* numel, int nseg,
-                                 float* dst, void* stream) {
+// two kernels rather than one template, so that profiles and the kernel-route tests name each by its own name
+__global__ void multi_copy_kernel(const CopySegs g, float* __restrict__ dst) {
+  multi_segment<false>(g.src[blockIdx.y], dst + g.off[blockIdx.y], g.n[blockIdx.y]);
+}
+__global__ void multi_accumulate_kernel(const CopySegs g, float* __restrict__ dst) {
+  multi_segment<true>(g.src[blockIdx.y], dst + g.off[blockIdx.y], g.n[blockIdx.y]);
+}
+
+template <bool kAdd>
+static int multi_segments(const float* const* src, const long long* dst_off, const long long* numel, int nseg,
+                          float* dst, void* stream) {
   if (nseg <= 0) return B200NP_OK;
   if (!src || !dst_off || !numel || !dst) return B200NP_E_BADARG;
   for (int base = 0; base < nseg; base += kSegsPerLaunch) {
@@ -81,11 +109,20 @@ extern "C" int b200np_multi_copy(const float* const* src, const long long* dst_o
     }
     long long bx = (mx + 1023) / 1024;   // 256 threads x 4 elements
     if (bx > 64) bx = 64;
-    multi_copy_kernel<<<dim3((unsigned)bx, (unsigned)cnt), 256, 0, as_stream(stream)>>>(g, dst);
+    (kAdd ? multi_accumulate_kernel : multi_copy_kernel)<<<dim3((unsigned)bx, (unsigned)cnt), 256, 0,
+                                                            as_stream(stream)>>>(g, dst);
     int rc = launch_status();
     if (rc != B200NP_OK) return rc;
   }
   return B200NP_OK;
+}
+extern "C" int b200np_multi_copy(const float* const* src, const long long* dst_off, const long long* numel, int nseg,
+                                 float* dst, void* stream) {
+  return multi_segments<false>(src, dst_off, numel, nseg, dst, stream);
+}
+extern "C" int b200np_multi_accumulate(const float* const* src, const long long* dst_off, const long long* numel,
+                                       int nseg, float* dst, void* stream) {
+  return multi_segments<true>(src, dst_off, numel, nseg, dst, stream);
 }
 
 // ------------------------------------------------------------------------------------------------
